@@ -29,13 +29,19 @@ one pass of the whole read set through the hot path, as a sequence of 64-Mbase b
           more than 2^32 super-read bases = an index of several parts, 15 kbp reads, k = 17); not the
           metric's configuration, reported in DESIGN.md.
   --workload lookup : configs[4], k-mer queries against a 1 Gbp suffix array.
+  --dump-outputs DIR : after the timed steps, the coords rows the device-timed path returned in its last step, for a
+          fixed, seeded sample of the reads, as DIR/<name>.npy (OutputDump); the inputs are the same from run to run,
+          so two builds can be compared output for output.  Not offered for --workload lookup: that microbench
+          times one kernel on random queries, and its results are checked against the oracle by the test suite.
 """
 import argparse
 import ctypes as C
 import json
 import os
+import queue
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -75,7 +81,15 @@ def parse_args():
     ap.add_argument("--lookup-n", type=float, default=1e9)
     ap.add_argument("--lookup-queries", type=float, default=1e9)
     ap.add_argument("--lookup-k", type=int, default=17)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the rows the device-timed path returned in its last step (a seeded sample of the reads, at most "
+                         "64 MB) as DIR/<name>.npy; rank 0's shard when --gpus > 1")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "mega_reads"):
+        ap.error("--dump-outputs: only the GPU path of the mega_reads workload")
+    return args
 
 
 def data_files(args):
@@ -87,7 +101,7 @@ def data_files(args):
                  read_len=15000, error=0.15, sr_cov=1.4, repeat_frac=0.2, seed=45,
                  mer=17)                       # mega_reads_assemble.sh:10 (MER=17): at 15 a random mer has ~8 chance matches in 8.7 G bases
     tag = "g%d_c%g_s%d_r%g_l%d" % (w["genome"], w["coverage"], w["seed"], w["repeat_frac"], w["read_len"])
-    d = os.path.join(os.environ.get("MR_BENCH_DIR", "/tmp/pacbio_b200_bench"), tag)
+    d = os.path.join(os.environ.get("MR_BENCH_DIR", os.path.join(tempfile.gettempdir(), "pacbio_b200_bench")), tag)
     prefix = os.path.join(d, "synth")
     done = prefix + ".done"
     rank = int(os.environ.get("RANK", "0"))
@@ -537,6 +551,104 @@ def cli_run(w, files, total_bases, host_threads, gpus=1):
 
 
 # --------------------------------------------------------------------------------------------------
+# --dump-outputs
+# --------------------------------------------------------------------------------------------------
+DUMP_FIELDS = ("rs", "re", "qs", "qe", "nb_mers", "pb_cons", "sr_cons", "pb_cover", "sr_cover", "ql", "sr", "rn", "use_bwd",
+               "stretch", "offset", "avg_err", "info_len", "start_node", "end_node", "lstart", "lprev", "lpath", "lunitigs",
+               "component")
+DUMP_BYTES = 63 << 20                   # array bytes; the .npy headers stay well inside the 64 MB the option promises
+
+
+def _ranges(start, count):
+    """start[i], start[i] + 1, ..., start[i] + count[i] - 1 for every i, one range after the other."""
+    return np.repeat(start - (np.cumsum(count) - count), count) + np.arange(int(count.sum()))
+
+
+class OutputDump:
+    """The results of one step, for a fixed sample of the reads: an eighth of them drawn with a fixed seed, or fewer
+    (those drawn first) when their rows would pass DUMP_BYTES.  write() leaves in DIR
+      read_index.npy             the sampled reads, by position in the read file
+      read_rows.npy              coords rows of each sampled read
+      <field>.npy                every row field of mr_result_view (DUMP_FIELDS), rows of the sampled reads in read order;
+                                 the overlap graph's fields only when the step ran the graph
+      kmers_info.npy, bases_info.npy   the info lists of those rows one after the other, info_len entries each
+    all float64, which holds every value of these int32 / uint32 / uint8 / double fields exactly.
+    put() hands a result over; its rows are copied out on a thread of its own, so the next batch's kernels do not wait
+    for the copy, and the result is freed there as soon as they are.  Freeing a result returns its page-locked slab to
+    the context's pool; a copy takes about a millisecond of host time and a batch several milliseconds of GPU time, so
+    the slab is normally back before the next batch asks for one and the step allocates no new page-locked memory."""
+
+    def __init__(self, nreads, view, free, seed=0):
+        self.view, self.free = view, free
+        self.draw = np.random.default_rng(seed).permutation(nreads)          # read r is drawn draw[r]-th
+        self.pick = np.flatnonzero(self.draw < max(1, nreads // 8))
+        self.parts, self.errors = [], []
+        self.queue = queue.Queue()
+        self.thread = threading.Thread(target=self._drain, daemon=True)
+        self.thread.start()
+
+    def put(self, first_read, result):
+        """result: what the batch whose first read is first_read returned."""
+        self.queue.put((first_read, result))
+
+    def _drain(self):
+        while True:
+            item = self.queue.get()
+            if item is None:
+                return
+            try:
+                if not self.errors:
+                    self.parts.append((item[0], self._take(*item)))
+            except Exception as e:                               # noqa: BLE001  (raised again by write())
+                self.errors.append(e)
+            finally:
+                self.free(item[1])
+
+    def _take(self, first, result):
+        v = self.view(result)
+        nr, n = int(v.nreads), int(v.ncoords)
+        lo, hi = np.searchsorted(self.pick, [first, first + nr])
+        reads = self.pick[lo:hi]
+        rc = np.ctypeslib.as_array(v.read_coords, shape=(nr + 1,)).astype(np.int64)
+        start, count = rc[reads - first], rc[reads - first + 1] - rc[reads - first]
+        part = {"read_index": reads, "read_rows": count}
+        if n == 0:
+            return dict(part, **{f: np.zeros(0) for f in DUMP_FIELDS + ("kmers_info", "bases_info")})
+        rows = _ranges(start, count)
+        for f in DUMP_FIELDS:
+            if getattr(v, f):
+                part[f] = np.ctypeslib.as_array(getattr(v, f), shape=(n,))[rows]
+        off = np.ctypeslib.as_array(v.info_off, shape=(n,))[rows].astype(np.int64)
+        length = part["info_len"].astype(np.int64)
+        at = _ranges(off, length)
+        total = int((off + length).max()) if len(at) else 0
+        for f in ("kmers_info", "bases_info"):
+            part[f] = np.ctypeslib.as_array(getattr(v, f), shape=(total,))[at] if total else np.zeros(0)
+        return part
+
+    def write(self, path):
+        self.queue.put(None)
+        self.thread.join()
+        if self.errors:
+            raise self.errors[0]
+        parts = [p for _, p in sorted(self.parts, key=lambda x: x[0])]
+        out = {k: np.concatenate([p[k] for p in parts]).astype(np.float64) for k in parts[0] if all(k in p for p in parts)}
+        rows, info = out["read_rows"].astype(np.int64), out["info_len"].astype(np.int64)
+        row_fields = [k for k in out if k in DUMP_FIELDS]
+        info_of_read = np.bincount(np.repeat(np.arange(len(rows)), rows), weights=info, minlength=len(rows))
+        nbytes = 8 * (2 + len(row_fields) * rows + 2 * info_of_read)
+        first = np.argsort(self.draw[out["read_index"].astype(np.int64)])
+        keep = np.zeros(len(rows), bool)
+        keep[first[np.cumsum(nbytes[first]) <= DUMP_BYTES]] = True
+        keep_row = np.repeat(keep, rows)
+        keep_info = np.repeat(keep_row, info)
+        os.makedirs(path, exist_ok=True)
+        for k, a in out.items():
+            mask = keep if k in ("read_index", "read_rows") else keep_row if k in row_fields else keep_info
+            np.save(os.path.join(path, k + ".npy"), a[mask])
+
+
+# --------------------------------------------------------------------------------------------------
 # our arm
 # --------------------------------------------------------------------------------------------------
 def ours(args, w, files):
@@ -636,19 +748,21 @@ def ours(args, w, files):
         hs = np.ctypeslib.as_array(ps, shape=(nr.value + 1,))
         dev.append((torch.from_numpy(hc).cuda(), torch.from_numpy(hm).cuda(), torch.from_numpy(hs.astype(np.int64)).cuda(), hs.copy(), nr.value))
     stream = torch.cuda.ExternalStream(L.mr_context_stream(ctx))
+    first_read = np.cumsum([0] + [d[4] for d in dev])
 
     phase = {}
     counters = dict(lookups=0, tails=0, hits=0, groups=0, coords=0, lists=0, buckets=0)
 
     import threading
 
-    def device_lane(lane, collect, errors):
+    def device_lane(lane, collect, errors, dump):
         # one thread per context: batches lane, lane + nstreams, ... (the C call releases the GIL)
         c = ctxs[lane]
         lnames = (C.c_char_p * 32)(); lsecs = (C.c_double * 32)()
         ph, cn = {}, dict(lookups=0, tails=0, hits=0, groups=0, coords=0, lists=0, buckets=0)
         try:
-            for dc, dm, ds, hs, nr in dev[lane::nstreams]:
+            for b in range(lane, nbatches, nstreams):
+                dc, dm, ds, hs, nr = dev[b]
                 out = C.c_void_p()
                 rc = L.mr_align_batch_device_packed(c, idx, C.cast(params, C.POINTER(api.Params)), C.c_void_p(dc.data_ptr()),
                                                     C.c_void_p(dm.data_ptr()), C.c_void_p(ds.data_ptr()),
@@ -663,15 +777,18 @@ def ours(args, w, files):
                     L.mr_result_get(out, C.byref(v))
                     cn["lookups"] += v.n_kmers_looked_up; cn["tails"] += v.n_tail_entries; cn["hits"] += v.n_hits
                     cn["groups"] += v.n_groups; cn["coords"] += v.ncoords; cn["lists"] += v.n_lists; cn["buckets"] += v.n_buckets
-                L.mr_result_free(out)
+                if dump is not None:
+                    dump.put(int(first_read[b]), out)
+                else:
+                    L.mr_result_free(out)
         except Exception as e:                       # noqa: BLE001
             errors.append(e)
         return ph, cn
 
-    def device_step(collect):
+    def device_step(collect, dump=None):
         errors, results = [], [None] * nstreams
         def run(lane):
-            results[lane] = device_lane(lane, collect, errors)
+            results[lane] = device_lane(lane, collect, errors, dump)
         threads = [threading.Thread(target=run, args=(lane,)) for lane in range(1, nstreams)]
         for t in threads:
             t.start()
@@ -693,10 +810,18 @@ def ours(args, w, files):
     sampler = ClockSampler(local_rank)
     sampler.start()
     launches0 = sum(L.mr_context_launches(c_) for c_ in ctxs)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        def view(result):
+            v = api.ResultView()
+            if L.mr_result_get(result, C.byref(v)) != 0:
+                raise RuntimeError("mr_result_get failed")
+            return v
+        dump = OutputDump(int(first_read[-1]), view, L.mr_result_free)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
-    for _ in range(args.steps):
-        device_step(True)
+    for step in range(args.steps):
+        device_step(True, dump if step == args.steps - 1 else None)
     e1.record(stream)
     torch.cuda.synchronize()
     barrier(dist)
@@ -725,6 +850,8 @@ def ours(args, w, files):
     e2e_value = job_bases * args.steps / e2e_s_max
     st_align, st_format = C.c_double(), C.c_double()
     H.mrh_tool_stage_seconds(tool, C.byref(st_align), C.byref(st_format))
+    if dump is not None:
+        dump.write(args.dump_outputs)
 
     # ---- roofline of the dominant kernel ---------------------------------------------------------------
     # Phase timers are CUDA events recorded on the library's own stream around each phase; the

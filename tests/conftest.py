@@ -21,7 +21,7 @@ def port():
 def ref():
     from oracle_lib import Ref, have_ref
     if not have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref not built (it is compiled from the original project's sources, see oracle/Makefile)")
     return Ref()
 
 

@@ -225,6 +225,78 @@ def test_bench_workload_shapes(tmp_path, monkeypatch):
     assert "configs[1]" in bench.config_dict(b, w2)["workload"]
 
 
+def test_bench_output_dump(tmp_path, monkeypatch):
+    """bench.py --dump-outputs (bench.OutputDump) on results of two batches built here: the rows and info lists of a
+    seeded sample of the reads, in read order, as float64; the same files from run to run; every result freed; fewer
+    reads (the first drawn) when the rows would pass the size budget."""
+    import ctypes as C
+    import pacbio_b200.api as api
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(8)
+    nreads, cut = 200, 120
+    rows_of = rng.integers(0, 6, size=nreads)
+    keep_alive, batches = [], []
+    for first, nr in ((0, cut), (cut, nreads - cut)):
+        cnt = rows_of[first:first + nr]
+        n = int(cnt.sum())
+        v = api.ResultView()
+        v.nreads, v.ncoords = nr, n
+        arrays = {"read_coords": np.concatenate([[0], np.cumsum(cnt)]).astype(np.uint64)}
+        for f, t in api.ResultView._fields_:
+            if f in bench.DUMP_FIELDS and f not in ("info_len", "lstart", "lprev", "lpath", "lunitigs", "component"):
+                dt = {api.u8p: np.uint8, api.i32p: np.int32, api.u32p: np.uint32, api.f64p: np.float64}[t]
+                arrays[f] = (rng.integers(0, 250, size=n) + (rng.random(n) if dt is np.float64 else 0)).astype(dt)
+        arrays["info_len"] = rng.integers(0, 4, size=n).astype(np.uint32)
+        arrays["info_off"] = (np.cumsum(arrays["info_len"]) - arrays["info_len"])[rng.permutation(n)].astype(np.uint64)
+        tot = int(arrays["info_len"].sum()) + 1
+        arrays["kmers_info"], arrays["bases_info"] = rng.integers(-9, 99, size=tot).astype(np.int32), rng.integers(0, 99, size=tot).astype(np.int32)
+        for f, a in arrays.items():
+            setattr(v, f, a.ctypes.data_as(dict(api.ResultView._fields_)[f]))
+        keep_alive.append(arrays)
+        batches.append((first, v))
+
+    def run(path):
+        freed = []
+        d = bench.OutputDump(nreads, view=lambda h: h, free=freed.append)
+        for first, v in reversed(batches):                  # batches may come back in any order
+            d.put(first, v)
+        d.write(str(path))
+        assert sorted(map(id, freed)) == sorted(id(v) for _, v in batches)
+        return {f[:-4]: np.load(os.path.join(path, f)) for f in os.listdir(path)}
+
+    got = run(tmp_path / "a")
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert "lpath" not in got                                # graph fields: not computed, not written
+    reads = got["read_index"].astype(np.int64)
+    assert len(reads) == nreads // 8 and np.all(np.diff(reads) > 0)
+    assert np.array_equal(got["read_rows"], rows_of[reads])
+    want = {k: [] for k in got if k not in ("read_index", "read_rows")}
+    for r in reads:
+        a, first = (keep_alive[0], 0) if r < cut else (keep_alive[1], cut)
+        rc = a["read_coords"].astype(np.int64)
+        for row in range(rc[r - first], rc[r - first + 1]):
+            for k in want:
+                if k in ("kmers_info", "bases_info"):
+                    o, n = int(a["info_off"][row]), int(a["info_len"][row])
+                    want[k].extend(a[k][o:o + n].tolist())
+                else:
+                    want[k].append(a[k][row])
+    for k, w in want.items():
+        assert np.array_equal(got[k], np.array(w, dtype=np.float64)), k
+    again = run(tmp_path / "b")
+    assert all(np.array_equal(got[k], again[k]) for k in got)
+    # a budget for about half of the sample: the reads drawn first stay, with all their rows
+    row_bytes = 8 * (sum(1 for k in got if k in bench.DUMP_FIELDS) + 2 * got["info_len"].mean())
+    monkeypatch.setattr(bench, "DUMP_BYTES", int(row_bytes * got["read_rows"].sum() / 2))
+    small = run(tmp_path / "c")
+    assert 0 < len(small["read_index"]) < len(reads)
+    draw = np.random.default_rng(0).permutation(nreads)
+    kept = set(small["read_index"].astype(int).tolist())
+    assert max(draw[list(kept)]) < min(draw[[r for r in reads if r not in kept]])
+    assert len(small["rs"]) == small["read_rows"].sum()
+
+
 def test_fixed_point_formatter_prints_what_printf_prints():
     """The mega-read lines carry "%.2f" / "%.4f" doubles (overlap_graph.cc:285-290); the host formatter prints
     them with its own exact routine instead of glibc's (13x faster): same strings on 2e6 operands."""
