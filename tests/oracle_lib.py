@@ -252,6 +252,38 @@ def read_fasta(path):
     return names, seqs
 
 
+def canon_rows(cint, cdbl, info_off, kinfo, binfo):
+    """Coords rows as comparable tuples: integers exact, doubles by their bit pattern (float.hex), each row's
+    kmers_info / bases_info slice."""
+    rows = []
+    for j in range(len(cint)):
+        lo, hi = info_off[j], info_off[j + 1]
+        rows.append((tuple(int(x) for x in cint[j]), tuple(float(x).hex() for x in cdbl[j]),
+                     tuple(kinfo[lo:hi].tolist()), tuple(binfo[lo:hi].tolist())))
+    return rows
+
+
+def oracle_rows(o):
+    """canon_rows of one read's result from a checker's align_read."""
+    return canon_rows(o["cint"], o["cdbl"], o["info_off"], o["kinfo"], o["binfo"])
+
+
+def device_rows(res, r, read_len):
+    """canon_rows of read r of a pacbio_b200 Result, laid out as the checkers' align_read lays them out
+    (cint = rs, re, qs, qe, nb_mers, pb_cons, sr_cons, pb_cover, sr_cover, read length, ql, rn, sr, use_bwd)."""
+    rr = list(res.rows(r))
+    if not rr:
+        return []
+    g_int = np.stack([res.rs[rr], res.re[rr], res.qs[rr], res.qe[rr], res.nb_mers[rr], res.pb_cons[rr],
+                      res.sr_cons[rr], res.pb_cover[rr], res.sr_cover[rr], np.full(len(rr), read_len), res.ql[rr],
+                      res.rn[rr], res.sr[rr], res.use_bwd[rr]], axis=1).astype(np.int64)
+    g_dbl = np.stack([res.stretch[rr], res.offset[rr], res.avg_err[rr]], axis=1)
+    g_off = np.concatenate([[0], np.cumsum(res.info_len[rr])]).astype(np.int64)
+    g_k = np.concatenate([res.info(i)[0] for i in rr])
+    g_b = np.concatenate([res.info(i)[1] for i in rr])
+    return canon_rows(g_int, g_dbl, g_off, g_k, g_b)
+
+
 def records(path_or_text, is_text=False):
     """Parse create_mega_reads / compact jf_aligner output into {read header: sorted tuple of lines}."""
     text = path_or_text if is_text else open(path_or_text).read()

@@ -5,7 +5,7 @@ import os
 import numpy as np
 import pytest
 
-from oracle_lib import gen_synth, read_fasta
+from oracle_lib import device_rows, gen_synth, oracle_rows, read_fasta
 
 pytestmark = [pytest.mark.gpu, pytest.mark.timeout(600)]
 
@@ -178,15 +178,6 @@ def test_lookup_at_scale_matches_reference_psa_search(ctx, port, tmpdir_session,
     assert int((gn > 0).sum()) >= nq // 4           # every k-mer sampled on the text's own strand is found (the search is strand specific)
 
 
-def _canon(cint, cdbl, info_off, kinfo, binfo):
-    rows = []
-    for j in range(len(cint)):
-        lo, hi = info_off[j], info_off[j + 1]
-        rows.append((tuple(int(x) for x in cint[j]), tuple(float(x).hex() for x in cdbl[j]),
-                     tuple(kinfo[lo:hi].tolist()), tuple(binfo[lo:hi].tolist())))
-    return rows
-
-
 @pytest.mark.parametrize("forward,window", [(True, 1), (False, 1), (True, 3), (False, 2)])
 def test_align_stages_match_oracle(case, ctx, port, forward, window):
     """hit lists, both chains and coords rows of every (read, super-read) pair against the oracle port; window > 1 is
@@ -212,6 +203,8 @@ def test_align_stages_match_oracle(case, ctx, port, forward, window):
     ctx.keep_taps(True)
     res = ctx.align(case["idx"], sub, p)
     ctx.keep_taps(False)
+    # the same reads without taps: single-hit groups and groups of up to 8 hits then take their own kernels
+    prod = ctx.align(case["idx"], sub, p)
     ap = port.aligner_create(case["hp"], unitigs_k=uk, forward=forward, window_size=window)
     total_coords = 0
     for r, s in enumerate(seqs):
@@ -225,18 +218,10 @@ def test_align_stages_match_oracle(case, ctx, port, forward, window):
         noff, nlis = int(o["groups"][:, 1:3].sum()), int(o["groups"][:, 3:5].sum())
         assert np.array_equal(res.tap_offsets[off0:off0 + noff], o["offsets"]), "hit lists of read %d" % r
         assert np.array_equal(res.tap_lis[lis0:lis0 + nlis], o["lis"]), "chains of read %d" % r
-        rr = list(res.rows(r))
-        assert len(rr) == len(o["cint"]), "coords count of read %d" % r
-        total_coords += len(rr)
-        g_int = np.stack([res.rs[rr], res.re[rr], res.qs[rr], res.qe[rr], res.nb_mers[rr], res.pb_cons[rr],
-                          res.sr_cons[rr], res.pb_cover[rr], res.sr_cover[rr], np.full(len(rr), len(s)), res.ql[rr],
-                          res.rn[rr], res.sr[rr], res.use_bwd[rr]], axis=1).astype(np.int64) if rr else np.zeros((0, 14), np.int64)
-        g_dbl = np.stack([res.stretch[rr], res.offset[rr], res.avg_err[rr]], axis=1) if rr else np.zeros((0, 3))
-        g_off = np.concatenate([[0], np.cumsum(res.info_len[rr])]).astype(np.int64)
-        g_k = np.concatenate([res.info(i)[0] for i in rr]) if rr else np.zeros(0, np.int32)
-        g_b = np.concatenate([res.info(i)[1] for i in rr]) if rr else np.zeros(0, np.int32)
-        assert _canon(g_int, g_dbl, g_off, g_k, g_b) == _canon(o["cint"], o["cdbl"], o["info_off"], o["kinfo"], o["binfo"]), \
-            "coords of read %d" % r
+        want = oracle_rows(o)
+        assert device_rows(res, r, len(s)) == want, "coords of read %d" % r
+        assert device_rows(prod, r, len(s)) == want, "coords of read %d without taps" % r
+        total_coords += len(want)
     assert total_coords > 20
     port.aligner_destroy(ap)
 
@@ -375,16 +360,7 @@ def test_max_match_coords_match_oracle(case, ctx, port):
     for r in range(n):
         o = port.align_read(ap, seqs[r])
         rr = list(res.rows(r))
-        assert len(rr) == len(o["cint"]), "coords count of read %d" % r
-        g_int = np.stack([res.rs[rr], res.re[rr], res.qs[rr], res.qe[rr], res.nb_mers[rr], res.pb_cons[rr],
-                          res.sr_cons[rr], res.pb_cover[rr], res.sr_cover[rr], np.full(len(rr), len(seqs[r])), res.ql[rr],
-                          res.rn[rr], res.sr[rr], res.use_bwd[rr]], axis=1).astype(np.int64) if rr else np.zeros((0, 14), np.int64)
-        g_dbl = np.stack([res.stretch[rr], res.offset[rr], res.avg_err[rr]], axis=1) if rr else np.zeros((0, 3))
-        g_off = np.concatenate([[0], np.cumsum(res.info_len[rr])]).astype(np.int64)
-        g_k = np.concatenate([res.info(i)[0] for i in rr]) if rr else np.zeros(0, np.int32)
-        g_b = np.concatenate([res.info(i)[1] for i in rr]) if rr else np.zeros(0, np.int32)
-        assert _canon(g_int, g_dbl, g_off, g_k, g_b) == _canon(o["cint"], o["cdbl"], o["info_off"], o["kinfo"], o["binfo"]), \
-            "coords of read %d" % r
+        assert device_rows(res, r, len(seqs[r])) == oracle_rows(o), "coords of read %d" % r
         extra += len(rr) - len(set(res.sr[rr].tolist()))
     assert extra > 0, "no secondary match was exercised"
     port.aligner_destroy(ap)
