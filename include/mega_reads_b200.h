@@ -229,7 +229,10 @@ int  mr_graph_batch(mr_context* ctx, const mr_params* params, const mr_result_vi
 
 /* parity tap: per-(read, super-read) hit lists and chains of the last batch, in the layout of
  * tests/oracle_lib.py (groups[g] = {read, sr, n_fwd, n_bwd, lis_fwd, lis_bwd}); only filled when
- * mr_context_keep_taps(ctx, 1) was called before the batch. */
+ * mr_context_keep_taps(ctx, 1) was called before the batch.  With max_match the lists are the
+ * ones the discard loop ends with: the hits of the chains it removed are gone from n_fwd / n_bwd
+ * and the offsets, and each chain is the list's latest one (the chain that failed the filters, or
+ * empty), as indices into that shortened list.  Not available with a fine pass (MR_EINVAL). */
 int  mr_context_keep_taps(mr_context* ctx, int on);
 int  mr_result_taps(const mr_result* r, uint64_t* ngroups, const int64_t** groups,
                     uint64_t* noffsets, const int32_t** offsets, uint64_t* nlis, const uint32_t** lis);

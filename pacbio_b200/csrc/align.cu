@@ -1635,17 +1635,21 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
   MR_TRY(download_rows(ctx, ws, res.get(), fin, nreads, S, info_total, graph ? &GA : nullptr));
 
   // ---- parity taps: (read, super-read) hit lists and both chains, rows sorted by (read, sr) ------
+  // (--max-match: the lists after every discard, i.e. without the hits of the emitted chains that were removed)
   if(taps && G) {
     std::vector<uint64_t> hk(H), hp(H), hg(G + 1);
     std::vector<uint2> hl(G);
     std::vector<uint32_t> hcf(H), hcb(H);
+    std::vector<uint8_t> hrem(p->max_match ? H : 0);
     MR_CUDA(ctx, cudaMemcpyAsync(hk.data(), skeys, H * 8, cudaMemcpyDeviceToHost, st));
     MR_CUDA(ctx, cudaMemcpyAsync(hp.data(), spays, H * 8, cudaMemcpyDeviceToHost, st));
     MR_CUDA(ctx, cudaMemcpyAsync(hg.data(), ws.group_start.p, (G + 1) * 8, cudaMemcpyDeviceToHost, st));
     MR_CUDA(ctx, cudaMemcpyAsync(hl.data(), ws.tap_lens.p, G * 8, cudaMemcpyDeviceToHost, st));
     MR_CUDA(ctx, cudaMemcpyAsync(hcf.data(), ws.tap_cf.p, H * 4, cudaMemcpyDeviceToHost, st));
     MR_CUDA(ctx, cudaMemcpyAsync(hcb.data(), ws.tap_cb.p, H * 4, cudaMemcpyDeviceToHost, st));
+    if(p->max_match) MR_CUDA(ctx, cudaMemcpyAsync(hrem.data(), ws.removed.p, H, cudaMemcpyDeviceToHost, st));
     MR_CUDA(ctx, ctx->wait(st));
+    auto kept = [&](uint64_t i) { return hrem.empty() || !hrem[i]; };
     std::vector<uint64_t> ord(G);
     for(uint64_t g = 0; g < G; ++g) ord[g] = g;
     std::sort(ord.begin(), ord.end(), [&](uint64_t a, uint64_t b) { return hk[hg[a]] < hk[hg[b]]; });
@@ -1653,13 +1657,13 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
       const uint64_t b = hg[g], e = hg[g + 1];
       if((uint32_t)hk[b] == iv.nseq_all) continue;        // a read's hits that belong to no super-read
       int64_t nf = 0, nbw = 0;
-      for(uint64_t i = b; i < e; ++i) ((int32_t)(uint32_t)(hp[i] >> 32) > 0 ? nf : nbw)++;
+      for(uint64_t i = b; i < e; ++i) if(kept(i)) ((int32_t)(uint32_t)(hp[i] >> 32) > 0 ? nf : nbw)++;
       const int64_t row[6] = { (int64_t)(hk[b] >> 32), (int64_t)(uint32_t)hk[b], nf, nbw, hl[g].x, hl[g].y };
       res->tap_groups.insert(res->tap_groups.end(), row, row + 6);
       for(int pass = 0; pass < 2; ++pass)
         for(uint64_t i = b; i < e; ++i) {
           const int32_t so = (int32_t)(uint32_t)(hp[i] >> 32);
-          if((so > 0) == (pass == 0)) { res->tap_offsets.push_back((int32_t)(uint32_t)hp[i]); res->tap_offsets.push_back(so); }
+          if(kept(i) && (so > 0) == (pass == 0)) { res->tap_offsets.push_back((int32_t)(uint32_t)hp[i]); res->tap_offsets.push_back(so); }
         }
       for(uint32_t t = 0; t < hl[g].x; ++t) res->tap_lis.push_back(hcf[b + t]);
       for(uint32_t t = 0; t < hl[g].y; ++t) res->tap_lis.push_back(hcb[b + t]);
@@ -1679,7 +1683,6 @@ static int align_checked(mr_context* ctx, mr_index* idx, const mr_params* p, con
   // an index is read-only once built: any context of its device may align against it
   if(idx->ctx->device != ctx->device) return ctx->fail(MR_EINVAL, "mr_align_batch: index lives on another device");
   if(p->window_size < 1) return ctx->fail(MR_EINVAL, "mr_align_batch: --window-size must be at least 1");
-  if(p->max_match && ctx->keep_taps) return ctx->fail(MR_EINVAL, "mr_align_batch: parity taps are not available with --max-match");
   if(p->fine_mer && ctx->keep_taps) return ctx->fail(MR_EINVAL, "mr_align_batch: parity taps are not available with a fine pass");
   if(p->fine_mer && (p->fine_mer < idx->m || p->fine_mer > idx->k))
     return ctx->fail(MR_EINVAL, "mr_align_batch: the fine mer must lie between the psa_min and the mer length the index was built with "

@@ -981,6 +981,11 @@ __global__ void __launch_bounds__(128) finish_warp_kernel(chain_args A) {
 // chain of the strictly-longer-forward-else-backward list is removed from its list, that list is
 // chained again and the group is evaluated again, until a row fails.  One warp per group out of
 // global scratch; successive chains of a group are stored back to back in its chain_pay slice.
+// TAPS (parity taps on): record the state the loop ends in, as the reference's --details prints it: each strand's
+// latest chain, numbered within that strand's hits not yet removed.  A strand loses hits only right before it is
+// chained again, so its latest numbering is the one of its final hit list.  (A kernel of its own: the taps' extra live
+// values would make the production kernel spill more.)
+template<bool TAPS>
 __global__ void __launch_bounds__(128) chain_maxmatch_kernel(chain_args A, uint8_t* __restrict__ removed, uint32_t* __restrict__ cursor) {
   const unsigned lane = threadIdx.x & 31;
   while(true) {
@@ -997,9 +1002,9 @@ __global__ void __launch_bounds__(128) chain_maxmatch_kernel(chain_args A, uint8
     for(uint32_t t = lane; t < N; t += 32) rem[t] = 0;
     __syncwarp();
     uint32_t len_f = 0, best_f = 0, len_b = 0, best_b = 0, used = 0;
-    chain_strand_global(A.pays + gs, N, false, A.cb, gs, A.a, A.b, A.C, len_f, best_f, nullptr, rem, A.window);
+    chain_strand_global(A.pays + gs, N, false, A.cb, gs, A.a, A.b, A.C, len_f, best_f, TAPS ? A.tap_sub : nullptr, rem, A.window);
     __syncwarp();
-    chain_strand_global(A.pays + gs, N, true, A.cb, gs, A.a, A.b, A.C, len_b, best_b, nullptr, rem, A.window);
+    chain_strand_global(A.pays + gs, N, true, A.cb, gs, A.a, A.b, A.C, len_b, best_b, TAPS ? A.tap_sub : nullptr, rem, A.window);
     __syncwarp();
     uint32_t* pprev = A.cb.pprev + gs;
     uint32_t* chain = A.cb.Lelt + gs;            // L is dead between chainings
@@ -1024,8 +1029,18 @@ __global__ void __launch_bounds__(128) chain_maxmatch_kernel(chain_args A, uint8
         for(uint32_t t = 0; t < dn; ++t) { rem[cur] = 1; cur = pprev[cur]; }
       }
       __syncwarp();
-      if(drop_fwd) chain_strand_global(A.pays + gs, N, false, A.cb, gs, A.a, A.b, A.C, len_f, best_f, nullptr, rem, A.window);
-      else         chain_strand_global(A.pays + gs, N, true, A.cb, gs, A.a, A.b, A.C, len_b, best_b, nullptr, rem, A.window);
+      if(drop_fwd) chain_strand_global(A.pays + gs, N, false, A.cb, gs, A.a, A.b, A.C, len_f, best_f, TAPS ? A.tap_sub : nullptr, rem, A.window);
+      else         chain_strand_global(A.pays + gs, N, true, A.cb, gs, A.a, A.b, A.C, len_b, best_b, TAPS ? A.tap_sub : nullptr, rem, A.window);
+      __syncwarp();
+    }
+    if(TAPS) {
+      if(lane == 0) {
+        A.tap_lens[g] = make_uint2(len_f, len_b);
+        uint32_t cur = best_f;
+        for(uint32_t t = 0; t < len_f; ++t) { A.tap_cf[gs + len_f - 1 - t] = A.tap_sub[gs + cur]; cur = pprev[cur]; }
+        cur = best_b;
+        for(uint32_t t = 0; t < len_b; ++t) { A.tap_cb[gs + len_b - 1 - t] = A.tap_sub[gs + cur]; cur = pprev[cur]; }
+      }
       __syncwarp();
     }
   }
@@ -1104,7 +1119,8 @@ int launch_chain(mr_context* ctx, chain_args A, dev_buf& lists) {
   MR_LAUNCHED(ctx);
   CHAIN_TRACE(ctx->stream, "classify");
   if(A.max_match) {
-    chain_maxmatch_kernel<<<ctx->sm_count * 8, 128, 0, ctx->stream>>>(A, A.removed, ctr + 30);
+    if(A.tap_lens) chain_maxmatch_kernel<true><<<ctx->sm_count * 8, 128, 0, ctx->stream>>>(A, A.removed, ctr + 30);
+    else            chain_maxmatch_kernel<false><<<ctx->sm_count * 8, 128, 0, ctx->stream>>>(A, A.removed, ctr + 30);
     MR_LAUNCHED(ctx);
     return MR_OK;
   }

@@ -77,7 +77,6 @@ int main(int argc, char* argv[]) {
   if(l_given && u_given) error("Switches [-u, --unitigs-sequences=path] and [-l, --unitigs-lengths=path] are mutually exclusive");
   if(argc - optind != 0) error("Requires exactly 0 argument.");
   if(!details_given && !coords_given) error("No output file given. Doing nothing ungracefully.");
-  if(details_given && P.max_match) error("[--details] is not available together with --max-match in this build");
   if(details_given && P.fine_mer) error("[--details] is not available together with -F in this build");
   if(P.window_size < 1) error("[--window-size] must be at least 1");
   if((l_given || u_given) && !k_given)
