@@ -227,6 +227,43 @@ int  mr_graph_batch(mr_context* ctx, const mr_params* params, const mr_result_vi
                     const uint32_t* path_ids, const uint64_t* path_off, uint32_t npaths,
                     const int32_t* unitig_len, uint32_t n_unitigs, mr_result** out);
 
+/* ---- mega-read records: replaces overlap_graph::thread's printing side, i.e. term_node_per_comp, trim_match,
+ *  tile_greedy / tile_maximal and print_mega_reads (overlap_graph.cc:61-299, overlap_graph.hpp:198-262), on the
+ *  device, over the rows and graph nodes a batch left there.
+ *
+ *  mr_unitigs: the k-unitig sequences of the -u file (misc.cc:11-37), uploaded once: `seq` holds every sequence
+ *  back to back as in the file, off[i] .. off[i + 1] is unitig i (n + 1 offsets).  Read-only once created; any
+ *  context of the same device may use it.                                                                     */
+typedef struct mr_unitigs mr_unitigs;
+int  mr_unitigs_create(mr_context* ctx, const char* seq, const uint64_t* off, uint32_t n, mr_unitigs** out);
+void mr_unitigs_destroy(mr_unitigs* u);
+
+/* the options of the printing side (create_mega_reads_cmdline.yaggo): -k, -O, -d, -L, -T, --trim */
+typedef struct mr_records_params {
+  uint32_t unitigs_k;          /* -k */
+  double   overlap_play;       /* -O 1.3 */
+  double   density;            /* -d 0.029 */
+  double   min_length;         /* -L 100 */
+  int32_t  tiling;             /* -T: 0 none, 1 greedy, 2 maximal, 3 weighted */
+  int32_t  trim;               /* --trim: 0 none, non-zero trims as `match` does */
+} mr_records_params;
+
+/* The create_mega_reads text records of the reads of `r`, in read order: for every read with at least one
+ *  mega-read a ">name" line, then one line per mega-read (numbers, unitig path, super-read length and, with
+ *  `u`, the spliced sequence).  `r` must be the latest result of `ctx` and carry the overlap graph
+ *  (mr_align_* with run_graph, or mr_graph_batch): the rows are read where that batch left them on the
+ *  device; any other result gives MR_EINVAL.  u == NULL: no sequence column (-l).  names: the reads' names
+ *  back to back, name_off[r] .. name_off[r + 1] for read r (nreads + 1 offsets).
+ *  MR_EINVAL also for the inputs the reference rejects while printing: a unitig id of a super-read name
+ *  that the -u file does not have, and a component root outside the read's rows (mr_last_error says which).
+ *  The text lives in pinned host memory owned by the returned object: mr_text_get gives its bytes, valid
+ *  until mr_text_free.                                                                                  */
+typedef struct mr_text mr_text;
+int  mr_records(mr_context* ctx, const mr_result* r, const mr_records_params* p, const mr_unitigs* u,
+                const char* names, const uint64_t* name_off, mr_text** out);
+int  mr_text_get(const mr_text* t, const char** bytes, uint64_t* size);
+void mr_text_free(mr_text* t);
+
 /* parity tap: per-(read, super-read) hit lists and chains of the last batch, in the layout of
  * tests/oracle_lib.py (groups[g] = {read, sr, n_fwd, n_bwd, lis_fwd, lis_bwd}); only filled when
  * mr_context_keep_taps(ctx, 1) was called before the batch.  With max_match the lists are the

@@ -49,6 +49,19 @@ class ResultView(C.Structure):
                 ("n_groups", C.c_uint64), ("n_lists", C.c_uint64), ("n_buckets", C.c_uint64)]
 
 
+class RecordsParams(C.Structure):
+    _fields_ = [("unitigs_k", C.c_uint32), ("overlap_play", C.c_double), ("density", C.c_double),
+                ("min_length", C.c_double), ("tiling", C.c_int32), ("trim", C.c_int32)]
+
+
+def records_params(unitigs_k, **kw):
+    """The printing options of create_mega_reads (-k, -O, -d, -L, -T as 0 none / 1 greedy / 2 maximal / 3 weighted, --trim)."""
+    p = RecordsParams(unitigs_k=unitigs_k, overlap_play=1.3, density=0.029, min_length=100.0, tiling=1, trim=0)
+    for k, v in kw.items():
+        setattr(p, k, v)
+    return p
+
+
 _lib = None
 
 
@@ -115,6 +128,14 @@ def lib():
     L.mr_result_free.argtypes = [C.c_void_p]
     L.mr_result_get.argtypes = [C.c_void_p, C.POINTER(ResultView)]
     L.mr_result_taps.argtypes = [C.c_void_p, u64p, C.POINTER(i64p), u64p, C.POINTER(i32p), u64p, C.POINTER(u32p)]
+    L.mr_graph_batch.argtypes = [C.c_void_p, C.POINTER(Params), C.POINTER(ResultView), u32p, u32p, u64p, C.c_uint32, i32p,
+                                 C.c_uint32, C.POINTER(C.c_void_p)]
+    L.mr_unitigs_create.argtypes = [C.c_void_p, C.c_char_p, u64p, C.c_uint32, C.POINTER(C.c_void_p)]
+    L.mr_unitigs_destroy.argtypes = [C.c_void_p]
+    L.mr_records.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(RecordsParams), C.c_void_p, C.c_char_p, u64p,
+                             C.POINTER(C.c_void_p)]
+    L.mr_text_get.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), u64p]
+    L.mr_text_free.argtypes = [C.c_void_p]
     _lib = L
     return L
 
@@ -275,12 +296,59 @@ class Context:
     def index(self, sr, psa_min, k, unitig_len=None):
         return Index(self, sr, psa_min, k, unitig_len)
 
-    def align(self, index, reads, params):
+    def align(self, index, reads, params, keep=False):
+        """keep: the Result holds on to the native result (for records()) until its close()."""
         out = C.c_void_p()
         starts = np.ascontiguousarray(reads.starts, dtype=np.uint64)
         self.check(self.L.mr_align_batch(self.h, index.h, C.byref(params), reads.bases.ctypes.data_as(C.c_void_p),
                                          _p(starts, u64p), reads.nreads, C.byref(out)))
-        return Result(self, out)
+        return Result(self, out, keep)
+
+    def graph(self, rows, read_len, path_ids, path_off, unitig_len, params):
+        """mr_graph_batch over rows the caller made: `rows` maps every coords column of ResultView (and read_coords,
+        kmers_info, bases_info) to a numpy array; path_ids / path_off is the unitig-path table rows["sr"] indexes.
+        The Result keeps its native object, so that records() can print it."""
+        dt = {u8p: np.uint8, i32p: np.int32, u32p: np.uint32, f64p: np.float64, u64p: np.uint64}
+        v = ResultView()
+        keep = []
+        for name, t in ResultView._fields_:
+            if name in rows:
+                a = np.ascontiguousarray(rows[name], dtype=dt[t])
+                if len(a) == 0:
+                    a = np.zeros(1, dtype=dt[t])
+                keep.append(a)
+                setattr(v, name, _p(a, t))
+        v.nreads = len(rows["read_coords"]) - 1
+        v.ncoords = int(rows["read_coords"][-1])
+        rl = np.ascontiguousarray(read_len, dtype=np.uint32)
+        ids = np.ascontiguousarray(path_ids if len(path_ids) else [0], dtype=np.uint32)
+        off = np.ascontiguousarray(path_off, dtype=np.uint64)
+        ul = np.ascontiguousarray(unitig_len, dtype=np.int32)
+        out = C.c_void_p()
+        self.check(self.L.mr_graph_batch(self.h, C.byref(params), C.byref(v), _p(rl, u32p), _p(ids, u32p), _p(off, u64p),
+                                         len(off) - 1, _p(ul, i32p), len(ul), C.byref(out)))
+        return Result(self, out, True)
+
+    def unitigs(self, seq, off):
+        """The k-unitig sequences on this context's device (mr_unitigs_create): seq bytes, off[n + 1]."""
+        return Unitigs(self, seq, off)
+
+    def records(self, result, names, params, unitigs=None):
+        """The create_mega_reads records of `result` (which must be this context's latest, kept with keep=True),
+        printed on the device (mr_records); unitigs: Unitigs for the sequence column (-u), None for -l."""
+        if result.h is None:
+            raise MrError("records() needs a Result that kept its native object (align(..., keep=True) or graph())")
+        enc = [n.encode() if isinstance(n, str) else bytes(n) for n in names]
+        off = np.concatenate([[0], np.cumsum([len(n) for n in enc])]).astype(np.uint64)
+        t = C.c_void_p()
+        self.check(self.L.mr_records(self.h, result.h, C.byref(params), unitigs.h if unitigs is not None else None,
+                                     b"".join(enc), _p(off, u64p), C.byref(t)))
+        try:
+            p, n = C.c_void_p(), C.c_uint64()
+            self.check(self.L.mr_text_get(t, C.byref(p), C.byref(n)))
+            return C.string_at(p, n.value) if n.value else b""
+        finally:
+            self.L.mr_text_free(t)
 
     def align_packed(self, index, reads, params):
         """Same as align(), through the packed entry point: the batch is packed on the host (mr_pack_reads) and
@@ -379,10 +447,24 @@ def _arr(ptr, n, dtype):
     return np.ctypeslib.as_array(ptr, shape=(n,)).copy()
 
 
-class Result:
-    """Copies the pinned result arrays into numpy and frees the native object."""
+class Unitigs:
+    def __init__(self, ctx, seq, off):
+        self.ctx = ctx
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        h = C.c_void_p()
+        ctx.check(ctx.L.mr_unitigs_create(ctx.h, bytes(seq), _p(off, u64p), len(off) - 1, C.byref(h)))
+        self.h = h
 
-    def __init__(self, ctx, h):
+    def close(self):
+        if self.h:
+            self.ctx.L.mr_unitigs_destroy(self.h)
+            self.h = None
+
+
+class Result:
+    """Copies the pinned result arrays into numpy and frees the native object (with keep: at close())."""
+
+    def __init__(self, ctx, h, keep=False):
         v = ResultView()
         ctx.check(ctx.L.mr_result_get(h, C.byref(v)))
         self.view_struct = None
@@ -405,7 +487,16 @@ class Result:
         self.tap_groups = _arr(pg, ng.value * 6, np.int64).reshape(-1, 6)
         self.tap_offsets = _arr(po, no.value * 2, np.int32).reshape(-1, 2)
         self.tap_lis = _arr(pl, nl.value, np.uint32)
-        ctx.L.mr_result_free(h)
+        self.ctx, self.h = ctx, None
+        if keep:
+            self.h = h
+        else:
+            ctx.L.mr_result_free(h)
+
+    def close(self):
+        if self.h:
+            self.ctx.L.mr_result_free(self.h)
+            self.h = None
 
     def rows(self, r):
         return range(int(self.read_coords[r]), int(self.read_coords[r + 1]))

@@ -84,6 +84,13 @@ static int download_rows(mr_context* ctx, mr_workspace& ws, mr_result* res, cons
   return MR_OK;
 }
 
+// Stamps a finished result; with a graph, mr_records may read its rows where they are until the next batch.
+static void remember_rows(mr_workspace& ws, mr_result* res, const graph_args* GA, uint64_t S, int max_rows) {
+  res->stamp = ++ws.stamp;
+  if(!GA) return;
+  ws.graph_stamp = res->stamp;
+  ws.last_graph = *GA; ws.last_rows = S; ws.last_max_rows = max_rows;
+}
 
 static const bool g_trace = getenv("MR_TRACE") != nullptr;
 #define MR_TRACE_MSG(...) do { if(g_trace) { fprintf(stderr, "[mr] " __VA_ARGS__); fputc('\n', stderr); fflush(stderr); } } while(0)
@@ -1219,6 +1226,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
   cudaStream_t st = ctx->stream;
   if(!ctx->ws) ctx->ws = new mr_workspace;
   mr_workspace& ws = *ctx->ws;
+  ws.graph_stamp = 0;                       // the rows of the previous result are overwritten from here on
   const index_view& iv = idx->view;
   const uint32_t k = iv.k;
   const uint64_t T = h_read_start[nreads];
@@ -1672,6 +1680,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
   timer.end();
   MR_CUDA(ctx, ctx->wait(st));
   MR_TRACE_MSG("batch done");
+  remember_rows(ws, res.get(), graph ? &GA : nullptr, S, max_rows);
   *out = res.release();
   return MR_OK;
 }
@@ -1798,6 +1807,7 @@ int mr_graph_batch(mr_context* ctx, const mr_params* p, const mr_result_view* ro
   MR_CUDA(ctx, cudaSetDevice(ctx->device));
   if(!ctx->ws) ctx->ws = new mr_workspace;
   mr_workspace& ws = *ctx->ws;
+  ws.graph_stamp = 0;
   cudaStream_t st = ctx->stream;
   const uint32_t nreads = rows->nreads;
   const uint64_t S = rows->ncoords, Sc = std::max<uint64_t>(S, 1);
@@ -1862,6 +1872,7 @@ int mr_graph_batch(mr_context* ctx, const mr_params* p, const mr_result_view* ro
   timer.end();
   MR_CUDA(ctx, ctx->wait(st));
   timer.collect();
+  remember_rows(ws, res.get(), &GA, S, max_rows);
   *out = res.release();
   return MR_OK;
 }

@@ -46,6 +46,29 @@ struct mr_staged {
   ~mr_staged() { if(ready) cudaEventDestroy(ready); }
 };
 
+// graph.cu
+struct graph_args {
+  uint32_t nreads;
+  const uint64_t* read_coords;
+  const uint32_t* read_len;
+  coords_soa c;
+  const int32_t *kinfo, *binfo;
+  const uint32_t* unitig_ids; const uint64_t* unitig_off; const int32_t* unitig_len;
+  uint32_t n_unitigs, unitigs_k;
+  double overlap_play, errors;
+  int bases;
+  int warp_max_rows;       // reads with more rows than this take the edge-list kernels instead of one warp (big_rows_threshold())
+  double *ord_s, *ord_e, *ord_err;   // reads with many rows: imp_s, imp_e, avg_err in node order
+  ulonglong2* ord_path;              // ... and the node's unitig path: x = offset into unitig_ids, y = length | reversed << 32
+  uint32_t*   edge_cnt;              // out-edges of the node at every order position (0 for the rows of other reads)
+  uint64_t*   edge_off;              // exclusive scan of edge_cnt: a node's slice of `edges`
+  int4*       edges;                 // { successor's order position, weight - common, unitigs added, 0 }
+  // outputs / scratch, one entry per row
+  uint8_t *start_node, *end_node;
+  int32_t *lstart, *lprev, *lpath, *lunitigs, *component, *uf_rank, *order;
+  double  *imp_s, *imp_e;
+};
+
 // Scratch that lives in the context and is reused from batch to batch.
 struct mr_workspace {
   dev_buf bases, codes, nmask, read_start, read_len, tile_read, tile_pos, tile_first, tile_cand, tile_tbase;
@@ -62,14 +85,23 @@ struct mr_workspace {
   dev_buf tap_lens, tap_cf, tap_cb, group_lists, chain_pay, removed, chainW;
   dev_buf scan_scratch;
   prim::sort_scratch sort;
+  // mr_records: where the latest result's rows and graph nodes are (its stamp, 0: none with a graph), and scratch
+  uint64_t stamp = 0, graph_stamp = 0;
+  graph_args last_graph;
+  uint64_t last_rows = 0;
+  int last_max_rows = 0;
+  dev_buf rec_cand, rec_i32, rec_f64, rec_info, rec_lines, rec_linf, rec_names, rec_text;
+  pinned_buf rec_names_host;
+  std::vector<pinned_buf*> text_pool;       // pinned slabs of mr_text, recycled like the result slabs
   std::vector<pinned_buf*> pinned_pool;     // result slabs are recycled: cudaMallocHost costs milliseconds
   std::mutex pool_mutex;                    // mr_result_free may run on another host thread than mr_align_batch
   std::vector<mr_staged*> staged_pool;      // device input buffers of staged batches, recycled (cudaMalloc synchronises the device)
-  ~mr_workspace() { for(auto p : pinned_pool) delete p; for(auto s : staged_pool) delete s; }
+  ~mr_workspace() { for(auto p : pinned_pool) delete p; for(auto p : text_pool) delete p; for(auto s : staged_pool) delete s; }
 };
 
 struct mr_result {
   mr_context* ctx = nullptr;
+  uint64_t stamp = 0;               // mr_workspace::stamp of the batch that made it
   pinned_buf* host = nullptr;       // one pinned slab holding every array of the view (from the context's pool)
   mr_result_view view;
   // taps
@@ -125,28 +157,6 @@ struct chain_args {
 };
 int launch_chain(mr_context* ctx, chain_args A, dev_buf& lists);
 
-// graph.cu
-struct graph_args {
-  uint32_t nreads;
-  const uint64_t* read_coords;
-  const uint32_t* read_len;
-  coords_soa c;
-  const int32_t *kinfo, *binfo;
-  const uint32_t* unitig_ids; const uint64_t* unitig_off; const int32_t* unitig_len;
-  uint32_t n_unitigs, unitigs_k;
-  double overlap_play, errors;
-  int bases;
-  int warp_max_rows;       // reads with more rows than this take the edge-list kernels instead of one warp (big_rows_threshold())
-  double *ord_s, *ord_e, *ord_err;   // reads with many rows: imp_s, imp_e, avg_err in node order
-  ulonglong2* ord_path;              // ... and the node's unitig path: x = offset into unitig_ids, y = length | reversed << 32
-  uint32_t*   edge_cnt;              // out-edges of the node at every order position (0 for the rows of other reads)
-  uint64_t*   edge_off;              // exclusive scan of edge_cnt: a node's slice of `edges`
-  int4*       edges;                 // { successor's order position, weight - common, unitigs added, 0 }
-  // outputs / scratch, one entry per row
-  uint8_t *start_node, *end_node;
-  int32_t *lstart, *lprev, *lpath, *lunitigs, *component, *uf_rank, *order;
-  double  *imp_s, *imp_e;
-};
 struct mr_workspace;
 int launch_graph(mr_context* ctx, mr_workspace& ws, graph_args a, uint64_t S, int max_rows);
 // rows per read above which the per-read kernels (coords order, overlap graph) use a CTA instead of a

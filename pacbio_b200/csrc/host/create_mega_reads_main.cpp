@@ -149,14 +149,22 @@ int main(int argc, char* argv[]) {
     mrh::dot_state dstate;
     dstate.errors = P.errors; dstate.bases = P.bases;
     mrh::text_buf dot_text;
+    // the records are printed on the device (mr_records); --dot needs the host formatter, which recomputes the
+    // graph's edges and carries the stream state of the --dot file
+    mrh::device_unitigs DU;
+    mrh::records_fn records;
+    const mr_records_params RP = mrh::records_params(G);
+    if(!dot_file) {
+      DU.upload(DS, U);
+      records = [&](mr_context* c, const mr_result* r, const mrh::read_batch& b) { return mrh::device_records(c, r, RP, DU.of(c), b.name); };
+    }
     const uint64_t nb = mrh::run_pipeline(DS, pacbio, P,
-      [&](const mr_result*, const mr_result_view& v, const mrh::read_batch& b, std::vector<mrh::text_buf>& parts, const mrh::emit_fn& emit) {
-        if(!dot_file) { mrh::format_mega_reads_mt(v, b, SR, U, G, fthreads, parts, &emit); return; }
+      [&](const mr_result*, const mr_result_view& v, const mrh::read_batch& b, std::vector<mrh::text_buf>& parts) {
         parts.resize(1);
         parts[0].clear(); dot_text.clear();
         mrh::format_mega_reads(v, b, 0, v.nreads, SR, U, G, parts[0], &dot_text, &dstate);
         if(fwrite(dot_text.data(), 1, dot_text.size(), dot_file) != dot_text.size()) throw std::runtime_error("write error on the --dot file");
-      }, out, fthreads);
+      }, out, fthreads, records);
     if(dot_file && fclose(dot_file) != 0) throw std::runtime_error("write error on the --dot file");
     const auto t2 = std::chrono::steady_clock::now();
     if(show_timing) std::cerr << "Starting create mega reads ... " << std::chrono::duration<double>(t2 - t1).count()

@@ -157,7 +157,9 @@ struct graph_options {
 };
 
 // Text records of create_mega_reads for reads [r0, r1) of a result (overlap_graph.cc:61-299,
-// overlap_graph.hpp:198-262): best terminal node per component, tiling, one line per mega-read.
+// overlap_graph.hpp:198-262): best terminal node per component, tiling, one line per mega-read.  The tools print
+// their records on the device (mr_records); this host formatter is the one for --dot, whose edges it recomputes,
+// and the reference the device printer is tested against.
 // dot: when not null, also the reference's --dot text for these reads (overlap_graph.hpp:189-196, overlap_graph.cc:49-50,
 // 133-146,271): one "digraph" per read with every node, every overlap edge (recomputed here from the rows: the device
 // keeps only what the longest paths need) and the edges of the printed paths in red.  dot_state carries the one
@@ -167,31 +169,9 @@ struct dot_state { bool first_node = true; double errors = 3.0; int bases = 0; }
 void format_mega_reads(const mr_result_view& v, const read_batch& batch, uint32_t r0, uint32_t r1,
                        const super_reads& sr, const unitigs& u, const graph_options& o, text_buf& out,
                        text_buf* dot = nullptr, dot_state* ds = nullptr);
-// same, fanned out over `threads` host threads; parts[0], parts[1], ... concatenated are the records
-// in read order (kept apart so that nobody has to copy hundreds of megabytes of text once more)
-// With `emit`: the batch is formatted slice by slice, emit(parts) consumes the text of each slice (host_common.cpp).
-typedef std::function<void(std::vector<text_buf>&)> emit_fn;
-void format_mega_reads_mt(const mr_result_view& v, const read_batch& batch, const super_reads& sr, const unitigs& u,
-                          const graph_options& o, unsigned threads, std::vector<text_buf>& parts, const emit_fn* emit = nullptr);
-
-// Debug / profiling aid: one batch's result rows + read names on disk (MR_DUMP_BATCH=<file> in the bench's
-// host path writes the first batch), read back by pacbio_b200/tools/format_replay to time the
-// formatting stage on any host without a GPU.
-struct result_dump {
-  mr_result_view view;                  // points into the vectors below
-  read_batch     batch;                 // names and starts only (no bases)
-  std::vector<uint64_t> u64[2];         // read_coords, info_off
-  std::vector<int32_t>  i32[12];        // rs re qs qe nb_mers lstart lprev lpath lunitigs component kmers_info bases_info
-  std::vector<uint32_t> u32[7];         // pb_cons sr_cons pb_cover sr_cover ql sr info_len
-  std::vector<uint8_t>  u8[4];          // rn use_bwd start_node end_node
-  std::vector<double>   f64[3];         // stretch offset avg_err
-};
-bool dump_result(const std::string& path, const mr_result_view& v, const read_batch& batch);
-bool load_result(const std::string& path, result_dump& d);
-
-// self test of the fixed-point number formatter behind the mega-read lines: `samples` pseudo-random doubles
-// (decimal grids, half-way points, binary fractions, wide exponent range), "%.2f" and "%.4f", against
-// the C library; returns the number of strings that differ (must be 0)
+// self test of the fixed-point number formatter behind the mega-read lines (records_common.hpp): `samples`
+// pseudo-random doubles (decimal grids, half-way points, binary fractions, wide exponent range), "%.2f" and
+// "%.4f", against the C library; returns the number of strings that differ (must be 0)
 uint64_t selftest_fixed_format(uint64_t samples, uint64_t seed);
 
 // jf_aligner coords records (jf_aligner.cc:41-70)

@@ -114,7 +114,7 @@ int main(int argc, char* argv[]) {
     if(details) for(auto c : DS.ctx) mr_context_keep_taps(c, 1);
     mrh::text_buf dtext;
     mrh::run_pipeline(DS, pacbio, P,
-      [&](const mr_result* r, const mr_result_view& v, const mrh::read_batch& b, std::vector<mrh::text_buf>& parts, const mrh::emit_fn&) {
+      [&](const mr_result* r, const mr_result_view& v, const mrh::read_batch& b, std::vector<mrh::text_buf>& parts) {
         parts.resize(1);
         mrh::format_coords(v, b, 0, v.nreads, SR, compact, !zero_match, parts[0]);
         if(details) {                      // single formatter thread: no lock needed

@@ -25,7 +25,7 @@ static const char* usage_text =
 int main(int argc, char* argv[]) {
   using namespace cmdline;
   bool k_given = false, l_given = false, u_given = false;
-  uint32_t k_mer = 0, threads = 1;
+  uint32_t k_mer = 0;
   std::string unitigs_lengths, unitigs_sequences, output;
   mr_params P;
   mr_params_default(&P);
@@ -45,7 +45,7 @@ int main(int argc, char* argv[]) {
     case ':': case '?': error("Unrecognized or incomplete option");
     case 'h': case O_USAGE: fputs(usage_text, stdout); return 0;
     case 'V': puts("b200-mega-reads 0.1"); return 0;
-    case 't': threads = to_uint32(optarg, "-t, --threads=uint32"); break;
+    case 't': (void)to_uint32(optarg, "-t, --threads=uint32"); break;     // accepted; the records are printed on the GPU
     case 'o': output = optarg; break;
     case O_DOT: error("[--dot] writing the overlap graph is not implemented in this build");
     case 'O': P.overlap_play = G.overlap_play = to_double(optarg, "-O, --overlap-play=double"); break;
@@ -94,7 +94,10 @@ int main(int argc, char* argv[]) {
     uint64_t max_rows = 1u << 20;
     if(const char* e = getenv("MR_BATCH_ROWS")) max_rows = strtoull(e, nullptr, 0);
     mrh::coords_batch b;
-    std::vector<mrh::text_buf> parts;
+    const mr_records_params RP = mrh::records_params(G);
+    mr_unitigs* DU = nullptr;
+    if(U.has_sequences() && mr_unitigs_create(ctx, U.fwd.data(), U.off.data(), (uint32_t)U.len.size(), &DU) != MR_OK)
+      throw std::runtime_error(std::string("mr_unitigs_create: ") + mr_last_error(ctx));
     while(in.next_batch(b, max_rows)) {
       const mr_result_view rows = b.view();
       mr_result* r = nullptr;
@@ -102,13 +105,17 @@ int main(int argc, char* argv[]) {
       if(mr_graph_batch(ctx, &P, &rows, b.read_len.data(), b.paths.unitig_ids.empty() ? &no_ids : b.paths.unitig_ids.data(),
                         b.paths.unitig_off.data(), (uint32_t)b.paths.name.size(), U.len.data(), (uint32_t)U.len.size(), &r) != MR_OK)
         throw std::runtime_error(std::string("mr_graph_batch: ") + mr_last_error(ctx));
-      mr_result_view v;
-      mr_result_get(r, &v);
-      mrh::format_mega_reads_mt(v, b.reads, b.paths, U, G, std::max(1u, threads), parts);
-      for(const auto& text : parts)
-        if(!text.empty() && fwrite(text.data(), 1, text.size(), out) != text.size()) throw std::runtime_error("write error on output file");
+      // the records are printed on the device, from the rows and the path table mr_graph_batch left there
+      mr_text* t = mrh::device_records(ctx, r, RP, DU, b.reads.name);
+      const char* text = nullptr;
+      uint64_t n = 0;
+      mr_text_get(t, &text, &n);
+      const bool ok = n == 0 || fwrite(text, 1, n, out) == n;
+      mr_text_free(t);
       mr_result_free(r);
+      if(!ok) throw std::runtime_error("write error on output file");
     }
+    mr_unitigs_destroy(DU);
     mr_context_destroy(ctx);
     if(out != stdout) fclose(out);
   } catch(std::exception& e) {

@@ -5,6 +5,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <algorithm>
 #include <map>
 #include <stdexcept>
 #include <sys/stat.h>
@@ -104,6 +105,7 @@ namespace {
 struct part {
   std::unique_ptr<read_batch> batch;
   mr_result* result = nullptr;
+  mr_text* text = nullptr;           // the part's records, when the device printed them
 };
 struct job {
   uint64_t seq = 0;                  // position in the input stream
@@ -129,17 +131,30 @@ struct record_writer {
       if(cur >= 0) { fd = d; at = cur; }
     }
   }
+  struct span { const char* p; size_t n; };
   bool write(const std::vector<text_buf>& parts) {
+    std::vector<span> sp;
+    for(const auto& t : parts) sp.push_back(span{ t.data(), t.size() });
+    return write(sp);
+  }
+  // one block of text, cut in pieces of at least 4 MB for the parallel writes
+  bool write(const char* p, size_t n) {
+    std::vector<span> sp;
+    const size_t piece = std::max<size_t>(n / 8 + 1, 4u << 20);
+    for(size_t o = 0; o < n; o += piece) sp.push_back(span{ p + o, std::min(piece, n - o) });
+    return write(sp);
+  }
+  bool write(const std::vector<span>& parts) {
     if(fd < 0) {
-      for(const auto& t : parts) if(!t.empty() && fwrite(t.data(), 1, t.size(), out) != t.size()) return false;
+      for(const auto& t : parts) if(t.n && fwrite(t.p, 1, t.n, out) != t.n) return false;
       return true;
     }
     std::vector<off_t> where(parts.size());
-    for(size_t i = 0; i < parts.size(); ++i) { where[i] = at; at += (off_t)parts[i].size(); }
+    for(size_t i = 0; i < parts.size(); ++i) { where[i] = at; at += (off_t)parts[i].n; }
     std::atomic<bool> ok(true);
     auto put = [&](size_t i) {
-      const char* p = parts[i].data();
-      size_t left = parts[i].size();
+      const char* p = parts[i].p;
+      size_t left = parts[i].n;
       off_t o = where[i];
       while(left) {
         const ssize_t w = pwrite(fd, p, left, o);
@@ -148,8 +163,8 @@ struct record_writer {
       }
     };
     std::vector<std::thread> th;
-    for(size_t i = 1; i < parts.size(); ++i) if(!parts[i].empty()) th.emplace_back(put, i);
-    if(!parts.empty() && !parts[0].empty()) put(0);
+    for(size_t i = 1; i < parts.size(); ++i) if(parts[i].n) th.emplace_back(put, i);
+    if(!parts.empty() && parts[0].n) put(0);
     for(auto& t : th) t.join();
     return ok;
   }
@@ -158,7 +173,7 @@ struct record_writer {
 }
 
 uint64_t run_pipeline(device_set& ds, const std::vector<std::string>& read_paths, const mr_params& params,
-                      const format_fn& format, FILE* out, unsigned host_threads) {
+                      const format_fn& format, FILE* out, unsigned host_threads, const records_fn& records) {
   // 32 Mbases per batch.  The library itself does better with 64 (bench.py's default: 9.8 against 9.1 Gbases/s on the
   // yeast shape, 0.84 against 0.66 on the human one -- fewer synchronisation points, twice the groups per launch of the
   // persistent chaining kernels), but the tools are bound by their reader (~2 Gbases/s), and page-locking the packed
@@ -299,7 +314,14 @@ uint64_t run_pipeline(device_set& ds, const std::vector<std::string>& read_paths
                                        from_slot ? slots[g][sj.slot].nmask : b->nmask.data(), b->start.data(), b->nreads(), &pt.result);
             if(from_slot) { int k = sj.slot; sj.slot = -1; free_slots[g]->push(std::move(k)); }    // (a batch that is split is retried from its own arrays)
           }
-          if(rc == MR_OK) { pt.batch = std::move(b); j.parts.push_back(std::move(pt)); continue; }
+          if(rc == MR_OK) {
+            if(records) {                       // printed on the device while the rows are still there
+              try { pt.text = records(ds.ctx[g], pt.result, *b); } catch(std::exception& e) { fail(e.what()); }
+            }
+            pt.batch = std::move(b);
+            j.parts.push_back(std::move(pt));
+            continue;
+          }
           if((rc == MR_ELIMIT || rc == MR_ENOMEM) && b->nreads() > 1) {
             const uint32_t half = b->nreads() / 2;
             std::unique_ptr<read_batch> lo(new read_batch), hi(new read_batch);
@@ -333,22 +355,32 @@ uint64_t run_pipeline(device_set& ds, const std::vector<std::string>& read_paths
       waiting.emplace(j.seq, std::move(j));
       for(auto it = waiting.find(next_seq); it != waiting.end(); it = waiting.find(++next_seq)) {
         for(auto& pt : it->second.parts) {
-          mr_result_view v;
-          mr_result_get(pt.result, &v);
-          for(auto& p : parts) p.clear();
-          uint64_t wrote_us = 0;
-          const emit_fn emit = [&](std::vector<text_buf>& ps) { const uint64_t w0 = now_us(); if(!writer.write(ps)) fail("write error on output file"); wrote_us += now_us() - w0; };
           const uint64_t t0 = now_us();
-          try { format(pt.result, v, *pt.batch, parts, emit); } catch(std::exception& e) { fail(e.what()); }
-          emit(parts);
-          busy_format_us += now_us() - t0 - wrote_us; busy_write_us += wrote_us;
+          bool ok = true;
+          if(pt.text) {
+            const char* p = nullptr;
+            uint64_t n = 0;
+            mr_text_get(pt.text, &p, &n);
+            ok = writer.write(p, n);
+            mr_text_free(pt.text);
+            busy_write_us += now_us() - t0;
+          } else if(!failed) {
+            mr_result_view v;
+            mr_result_get(pt.result, &v);
+            for(auto& p : parts) p.clear();
+            try { format(pt.result, v, *pt.batch, parts); } catch(std::exception& e) { fail(e.what()); }
+            const uint64_t t1 = now_us();
+            ok = failed || writer.write(parts);
+            busy_format_us += t1 - t0; busy_write_us += now_us() - t1;
+          }
+          if(!ok) fail("write error on output file");
           mr_result_free(pt.result);
           recycle(pt.batch);
         }
         waiting.erase(it);
       }
     }
-    for(auto& w : waiting) for(auto& pt : w.second.parts) mr_result_free(pt.result);   // only after an error
+    for(auto& w : waiting) for(auto& pt : w.second.parts) { mr_text_free(pt.text); mr_result_free(pt.result); }   // only after an error
     writer.finish();
   });
 
@@ -363,6 +395,43 @@ uint64_t run_pipeline(device_set& ds, const std::vector<std::string>& read_paths
             1e-6 * busy_read_us, 1e-6 * busy_upload_us, ds.ctx.size(), 1e-6 * busy_align_us, ds.ctx.size(), 1e-6 * busy_format_us, 1e-6 * busy_write_us);
   if(!error.empty()) throw std::runtime_error(error);
   return total_bases;
+}
+
+mr_text* device_records(mr_context* ctx, const mr_result* r, const mr_records_params& p, const mr_unitigs* u,
+                        const std::vector<std::string>& names) {
+  std::string all;
+  std::vector<uint64_t> off(1, 0);
+  off.reserve(names.size() + 1);
+  for(const auto& n : names) { all += n; off.push_back(all.size()); }
+  mr_text* t = nullptr;
+  if(mr_records(ctx, r, &p, u, all.data(), off.data(), &t) != MR_OK) throw std::runtime_error(mr_last_error(ctx));
+  return t;
+}
+
+void device_unitigs::upload(const device_set& ds, const unitigs& U) {
+  if(!U.has_sequences()) return;
+  for(mr_context* c : ds.ctx) {
+    const int d = mr_context_device(c);
+    if(std::find(device.begin(), device.end(), d) != device.end()) continue;
+    mr_unitigs* x = nullptr;
+    if(mr_unitigs_create(c, U.fwd.data(), U.off.data(), (uint32_t)U.len.size(), &x) != MR_OK)
+      throw std::runtime_error(std::string("mr_unitigs_create: ") + mr_last_error(c));
+    device.push_back(d);
+    u.push_back(x);
+  }
+}
+
+const mr_unitigs* device_unitigs::of(mr_context* ctx) const {
+  const int d = mr_context_device(ctx);
+  for(size_t i = 0; i < device.size(); ++i) if(device[i] == d) return u[i];
+  return nullptr;
+}
+
+mr_records_params records_params(const graph_options& g) {
+  mr_records_params p;
+  p.unitigs_k = g.k_len; p.overlap_play = g.overlap_play; p.density = g.density; p.min_length = g.min_length;
+  p.tiling = g.tiling; p.trim = g.trim;
+  return p;
 }
 
 } // namespace mrh

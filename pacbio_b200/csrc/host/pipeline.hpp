@@ -73,13 +73,30 @@ bool stage_batches();
 // adds per_device - 1 more contexts for every device of ds, sharing the device's index
 void add_streams(device_set& ds, unsigned per_device);
 
-// format(result, view, batch, parts, emit): leaves the batch's text in parts[] (written by the pipeline when it
-// returns) and / or hands it over piecewise through emit(parts) on the way (format_mega_reads_mt)
-typedef std::function<void(const mr_result*, const mr_result_view&, const read_batch&, std::vector<text_buf>&, const emit_fn&)> format_fn;
+// format(result, view, batch, parts): the batch's text in parts[], written by the pipeline when it returns (host
+// formatting, on the one formatter thread)
+typedef std::function<void(const mr_result*, const mr_result_view&, const read_batch&, std::vector<text_buf>&)> format_fn;
+// records(context, result, batch): the batch's text produced on the device (mr_records), called by the aligner
+// thread of `context` right after the batch is aligned, while its rows are still on the device.  When given, it
+// replaces `format` and the formatter thread only writes the text; it throws std::runtime_error on failure.
+typedef std::function<mr_text*(mr_context*, const mr_result*, const read_batch&)> records_fn;
 
 // runs the whole stream; returns the number of read bases processed
 // host_threads: workers of the reader (parsing, packing); 0 = as many as the box has, up to 16
 uint64_t run_pipeline(device_set& ds, const std::vector<std::string>& read_paths, const mr_params& params,
-                      const format_fn& format, FILE* out, unsigned host_threads = 0);
+                      const format_fn& format, FILE* out, unsigned host_threads = 0, const records_fn& records = records_fn());
+
+// mr_records over a batch of a tool: the reads' names as the C ABI takes them, errors as exceptions
+mr_text* device_records(mr_context* ctx, const mr_result* r, const mr_records_params& p, const mr_unitigs* u,
+                        const std::vector<std::string>& names);
+// the -u sequences on every device of ds (one upload per device, shared by its contexts); empty without -u
+struct device_unitigs {
+  std::vector<int> device;
+  std::vector<mr_unitigs*> u;
+  ~device_unitigs() { for(auto x : u) mr_unitigs_destroy(x); }
+  void upload(const device_set& ds, const unitigs& U);
+  const mr_unitigs* of(mr_context* ctx) const;
+};
+mr_records_params records_params(const graph_options& g);
 
 } // namespace mrh

@@ -7,12 +7,14 @@
 #include <stdexcept>
 
 #include "pipeline.hpp"
+#include "../records_common.hpp"
 
 namespace {
 struct tool {
   mrh::super_reads SR;
   mrh::unitigs     U;
   mrh::device_set  DS;
+  mrh::device_unitigs DU;                             // the -u sequences on the device
   mrh::graph_options G;
   mr_params        P;
   std::vector<std::unique_ptr<mrh::read_batch>> batches;
@@ -21,7 +23,6 @@ struct tool {
   uint64_t last_text_bytes = 0, last_d2h_bytes = 0, last_h2d_bytes = 0, last_coords = 0;
   uint64_t last_lookups = 0, last_hits = 0, last_groups = 0;
   double   last_align_s = 0, last_format_s = 0;       // busy time of the two pipeline stages
-  std::vector<mrh::text_buf> parts;                   // text buffers, kept between runs (no re-faulting of ~1 GB)
 };
 }
 
@@ -39,6 +40,7 @@ void* mrh_tool_create(const char* sr_fasta, const char* unitigs_path, int unitig
     t->P.unitigs_k = unitig_k;
     t->P.run_graph = 1;
     t->G.k_len = unitig_k;
+    t->DU.upload(t->DS, t->U);
     return t.release();
   } catch(std::exception& e) {
     if(err && err_cap) { strncpy(err, e.what(), err_cap - 1); err[err_cap - 1] = 0; }
@@ -100,8 +102,9 @@ const uint64_t* mrh_tool_batch_starts(void* p, uint64_t i, uint32_t* nreads) {
 }
 
 // One full pass over the loaded reads through the public path: mr_align_batch from host memory
-// (H2D inside), results back (D2H inside), text records formatted on `threads` host threads while
-// the next batch is already on the GPU (same two-stage overlap as the command line tools).
+// (H2D inside), results back (D2H inside), text records printed on the device (mr_records) right after each
+// batch and written by a second thread while the next batch is already on the GPU (the same stages as the
+// command line tools).  `threads` is accepted for compatibility; nothing is formatted on the host.
 // out_path may be null/empty (text is produced and dropped).  Returns read bases processed, <0 on error.
 // mrh_tool_run_range: the same over batches [first, first + count) only (bench.py's parity gate writes
 // the records of the reads the CPU reference was run on).
@@ -117,6 +120,7 @@ int64_t mrh_tool_run_range(void* p, unsigned threads, const char* out_path, uint
   // one aligner thread per context takes the next batch; results are formatted in batch order
   const size_t nb = (size_t)count;
   std::vector<mr_result*> done(nb, nullptr);
+  std::vector<mr_text*> texts(nb, nullptr);
   uint64_t bases_done = 0;
   std::vector<char> ready(nb, 0);
   std::mutex m;
@@ -126,33 +130,27 @@ int64_t mrh_tool_run_range(void* p, unsigned threads, const char* out_path, uint
   std::string error, align_error;
   std::thread formatter([&]() {
     mrh::background_thread();
-    std::vector<mrh::text_buf>& parts = t->parts;
     for(size_t i = 0; i < nb; ++i) {
       mr_result* r = nullptr;
+      mr_text* text = nullptr;
       {
         std::unique_lock<std::mutex> l(m);
         cv.wait(l, [&] { return ready[i] || stop; });
         if(!ready[i]) return;
-        r = done[i];
+        r = done[i]; text = texts[i];
       }
       const auto f0 = std::chrono::steady_clock::now();
       mrh::read_batch* b = t->batches[first + i].get();
       bases_done += b->bases.size();
       mr_result_view v;
       mr_result_get(r, &v);
-      if(const char* dump = getenv("MR_DUMP_BATCH")) {       // profiling aid: the first batch's rows on disk, once
-        static std::atomic<bool> dumped(false);
-        if(*dump && !dumped.exchange(true) && !mrh::dump_result(dump, v, *b)) fprintf(stderr, "MR_DUMP_BATCH: cannot write %s\n", dump);
-      }
-      try {
-        const mrh::emit_fn emit = [&](std::vector<mrh::text_buf>& ps) {
-          for(const auto& text : ps) {
-            if(out) fwrite(text.data(), 1, text.size(), out);
-            t->last_text_bytes += text.size();
-          }
-        };
-        mrh::format_mega_reads_mt(v, *b, t->SR, t->U, t->G, threads, parts, &emit);
-      } catch(std::exception& e) { error = e.what(); }
+      const char* bytes = nullptr;
+      uint64_t nbytes = 0;
+      mr_text_get(text, &bytes, &nbytes);
+      if(out && nbytes && fwrite(bytes, 1, nbytes, out) != nbytes) error = "write error on output file";
+      t->last_text_bytes += nbytes;
+      t->last_d2h_bytes += nbytes;
+      mr_text_free(text);
       t->last_h2d_bytes += (b->codes.size() + b->nmask.size() + b->nreads() + 1) * 8ULL;
       uint64_t info = 0;
       for(uint64_t c = 0; c < v.ncoords; ++c) info += v.info_len[c];
@@ -202,10 +200,19 @@ int64_t mrh_tool_run_range(void* p, unsigned threads, const char* out_path, uint
         mrh::read_batch* b = t->batches[first + it.i].get();
         const int rc = it.s ? mr_align_staged(t->DS.ctx[s], t->DS.idx[s], &t->P, it.s, &r)
                             : mr_align_batch_packed(t->DS.ctx[s], t->DS.idx[s], &t->P, b->codes.data(), b->nmask.data(), b->start.data(), b->nreads(), &r);
+        mr_text* text = nullptr;
+        std::string rec_error;
+        if(rc == MR_OK) {
+          try { text = mrh::device_records(t->DS.ctx[s], r, mrh::records_params(t->G), t->DU.of(t->DS.ctx[s]), b->name); }
+          catch(std::exception& e) { rec_error = e.what(); mr_result_free(r); }
+        }
         busy[s] += std::chrono::duration<double>(std::chrono::steady_clock::now() - a0).count();
         std::lock_guard<std::mutex> l(m);
-        if(rc != MR_OK) { if(align_error.empty()) align_error = mr_last_error(t->DS.ctx[s]); stop = true; cv.notify_all(); continue; }
-        done[it.i] = r; ready[it.i] = 1;
+        if(rc != MR_OK || !rec_error.empty()) {
+          if(align_error.empty()) align_error = rc != MR_OK ? mr_last_error(t->DS.ctx[s]) : rec_error;
+          stop = true; cv.notify_all(); continue;
+        }
+        done[it.i] = r; texts[it.i] = text; ready[it.i] = 1;
         cv.notify_all();
       }
     });
@@ -214,7 +221,7 @@ int64_t mrh_tool_run_range(void* p, unsigned threads, const char* out_path, uint
   for(auto& th : aligners) th.join();
   formatter.join();
   for(double b : busy) t->last_align_s = std::max(t->last_align_s, b);
-  for(size_t i = 0; i < nb; ++i) if(ready[i] && i >= formatted) mr_result_free(done[i]);   // only after an error
+  for(size_t i = 0; i < nb; ++i) if(ready[i] && i >= formatted) { mr_text_free(texts[i]); mr_result_free(done[i]); }   // only after an error
   if(out) fclose(out);
   if(!align_error.empty() || !error.empty()) { t->error = align_error.empty() ? error : align_error; return -1; }
   return (int64_t)bases_done;
@@ -256,6 +263,70 @@ int mrh_selftest_read_stream(const char* const* paths, unsigned npaths, uint64_t
   }
 }
 uint64_t mrh_selftest_fixed_format(uint64_t samples, uint64_t seed) { return mrh::selftest_fixed_format(samples, seed); }
+// The fixed-point formatter of the records (records_common.hpp) and printf, side by side: both strings of x with d
+// decimals; returns whether they are equal.
+int mrh_fixed_format_pair(double x, int d, char* mine, char* libc) {
+  const int n = mrfmt::fmt_fixed(mine, x, d);
+  mine[n] = 0;
+  snprintf(libc, mrfmt::kFixedMax + 8, "%.*f", d, x);
+  return strcmp(mine, libc) == 0;
+}
+// The device's std::sort port against std::sort on n elements whose keys (kind 0, 1: ints, compared as the greedy
+// and maximal tilings compare lpath and tiling_end; 2: doubles, as the weighted tiling compares weights) are keys[];
+// returns the number of positions where the two permutations differ.
+uint64_t mrh_selftest_sort(int kind, const double* keys, uint64_t n) {
+  std::vector<int> a(n), b(n);
+  for(uint64_t i = 0; i < n; ++i) a[i] = b[i] = (int)i;
+  auto run = [&](auto comp) { std::sort(a.begin(), a.end(), comp); mrfmt::std_sort(b.data(), (long)n, comp); };
+  if(kind == 0) run([&](int i, int j) { return (int)keys[j] < (int)keys[i]; });
+  else if(kind == 1) run([&](int i, int j) { return keys[i] < keys[j]; });
+  else run([&](int i, int j) { return keys[j] < keys[i]; });
+  uint64_t bad = 0;
+  for(uint64_t i = 0; i < n; ++i) bad += a[i] != b[i];
+  return bad;
+}
+// The host formatter (mrh::format_mega_reads, the reference of the device printer) over a result: the super-read
+// paths the result's rows index (CSR), the k-unitig lengths, the sequences (useq == NULL: -l), the reads' names and
+// lengths (read_start: nreads + 1 offsets) and the printing options.  *out: malloc'ed text (mrh_free).  Returns 0,
+// or -1 with the message the tools print in err.
+int mrh_format_records(const mr_result* r, const uint32_t* path_ids, const uint64_t* path_off, uint32_t npaths,
+                       const int32_t* ulen, uint32_t nu, const char* useq, const uint64_t* uoff,
+                       const char* names, const uint64_t* name_off, const uint64_t* read_start,
+                       const mr_records_params* p, char** out, uint64_t* size, char* err, size_t err_cap) {
+  try {
+    mr_result_view v;
+    if(mr_result_get(r, &v) != MR_OK || !v.lstart) throw std::runtime_error("the result has no overlap graph");
+    mrh::super_reads sr;
+    sr.unitig_off.assign(path_off, path_off + npaths + 1);
+    sr.unitig_ids.assign(path_ids, path_ids + path_off[npaths]);
+    mrh::unitigs u;
+    u.len.assign(ulen, ulen + nu);
+    if(useq) {
+      u.off.assign(uoff, uoff + nu + 1);
+      u.fwd.assign(useq, uoff[nu]);
+      u.rc.resize(u.fwd.size());
+      for(uint32_t i = 0; i < nu; ++i)
+        for(uint64_t j = 0, n = uoff[i + 1] - uoff[i]; j < n; ++j) u.rc[uoff[i] + j] = mrfmt::revcomp_base((unsigned char)useq[uoff[i] + n - 1 - j]);
+    }
+    mrh::read_batch b;
+    b.start.assign(read_start, read_start + v.nreads + 1);
+    for(uint32_t i = 0; i < v.nreads; ++i) b.name.emplace_back(names + name_off[i], name_off[i + 1] - name_off[i]);
+    mrh::graph_options o;
+    o.k_len = p->unitigs_k; o.overlap_play = p->overlap_play; o.density = p->density; o.min_length = p->min_length;
+    o.tiling = p->tiling; o.trim = p->trim;
+    mrh::text_buf text;
+    mrh::format_mega_reads(v, b, 0, v.nreads, sr, u, o, text);
+    *out = (char*)malloc(text.size() + 1);
+    if(!*out) throw std::bad_alloc();
+    if(text.size()) memcpy(*out, text.data(), text.size());
+    *size = text.size();
+    return 0;
+  } catch(std::exception& e) {
+    if(err && err_cap) { strncpy(err, e.what(), err_cap - 1); err[err_cap - 1] = 0; }
+    return -1;
+  }
+}
+void mrh_free(void* p) { free(p); }
 void mrh_tool_stage_seconds(void* p, double* align_s, double* format_s) {
   tool* t = (tool*)p; *align_s = t->last_align_s; *format_s = t->last_format_s;
 }
