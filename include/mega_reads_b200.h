@@ -264,6 +264,38 @@ int  mr_records(mr_context* ctx, const mr_result* r, const mr_records_params* p,
 int  mr_text_get(const mr_text* t, const char** bytes, uint64_t* size);
 void mr_text_free(mr_text* t);
 
+/* ---- jf_aligner coords records: replaces print_coords (jf_aligner.cc:41-70) on the device, over the rows a batch
+ *  left there.
+ *
+ *  mr_sr_names: what a coords line names a super-read by (frag_info's fwd.name / bwd.name, super_reads::row_name):
+ *  the FASTA header after '>' as it was read (names[name_off[s] .. name_off[s + 1])), and the unitig path as
+ *  mr_index_create takes it (path_ids[path_off[s] .. path_off[s + 1]), (id << 1) | (ori == 'R'); path_ids may be
+ *  NULL when every path is empty).  A backward row of a super-read with a path prints that path reversed, F and R
+ *  swapped, as "<id><F|R>" joined by '_'; any other row prints the header.  The tools build it from their
+ *  super-reads, whatever -l / -u say; for rows of mr_graph_batch it is built from the caller's path table that
+ *  their `sr` indexes.  Read-only once created; any context of the same device may use it.                    */
+typedef struct mr_sr_names mr_sr_names;
+int  mr_sr_names_create(mr_context* ctx, const char* names, const uint64_t* name_off, const uint32_t* path_ids,
+                        const uint64_t* path_off, uint32_t nseq, mr_sr_names** out);
+void mr_sr_names_destroy(mr_sr_names* s);
+
+/* the options of jf_aligner's printing: --compact (non-zero: the compact format, the tool's default) and -0 */
+typedef struct mr_coords_params {
+  int32_t compact;             /* ">N name" before a read's N rows; 0: the read's name before every row  */
+  int32_t zero_match;          /* -0: a read without rows still gets its ">0 name" line (compact format) */
+} mr_coords_params;
+
+/* The jf_aligner coords text of the reads of `r`, in read order: one line per row ("Rstart Rend Qstart Qend Nmers
+ *  Rcons Qcons Rcover Qcover Rlen Qlen Stretch Offset Err" as "%d %d %d %d %d %u %u %u %u %llu %u %g %g %g ", the
+ *  super-read's name, then " kmers:bases" per kmers_info entry), under a ">N name" line per read (compact) or
+ *  after the read's name and a blank (not compact).  The column header line is the caller's.  `r` must be the
+ *  latest result of `ctx`, from any entry point (mr_align_*, with or without run_graph, -F, --max-match,
+ *  --window-size, or mr_graph_batch); any other result gives MR_EINVAL, as do names made on another device and a
+ *  row whose super-read index is not below the names' nseq (mr_last_error says which).  names / name_off: the
+ *  reads' names as mr_records takes them.  The text comes back as mr_records' does (mr_text_get / mr_text_free). */
+int  mr_coords_records(mr_context* ctx, const mr_result* r, const mr_coords_params* p, const mr_sr_names* s,
+                       const char* names, const uint64_t* name_off, mr_text** out);
+
 /* parity tap: per-(read, super-read) hit lists and chains of the last batch, in the layout of
  * tests/oracle_lib.py (groups[g] = {read, sr, n_fwd, n_bwd, lis_fwd, lis_bwd}); only filled when
  * mr_context_keep_taps(ctx, 1) was called before the batch.  With max_match the lists are the

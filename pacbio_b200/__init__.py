@@ -3,5 +3,5 @@
 Only what the path needs lives here: csrc/ (CUDA kernels, C ABI, host tools), api.py (ctypes
 binding used by tests and bench), tools/ (synthetic input generator).
 """
-from .api import (Context, Index, MrError, Params, Reads, RecordsParams, Result, SuperReads, Unitigs, default_params, lib,  # noqa: F401
-                  records_params)
+from .api import (Context, CoordsParams, Index, MrError, Params, Reads, RecordsParams, Result, SrNames, SuperReads, Unitigs,  # noqa: F401
+                  default_params, lib, records_params)

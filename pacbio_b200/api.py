@@ -54,6 +54,10 @@ class RecordsParams(C.Structure):
                 ("min_length", C.c_double), ("tiling", C.c_int32), ("trim", C.c_int32)]
 
 
+class CoordsParams(C.Structure):
+    _fields_ = [("compact", C.c_int32), ("zero_match", C.c_int32)]
+
+
 def records_params(unitigs_k, **kw):
     """The printing options of create_mega_reads (-k, -O, -d, -L, -T as 0 none / 1 greedy / 2 maximal / 3 weighted, --trim)."""
     p = RecordsParams(unitigs_k=unitigs_k, overlap_play=1.3, density=0.029, min_length=100.0, tiling=1, trim=0)
@@ -134,6 +138,10 @@ def lib():
     L.mr_unitigs_destroy.argtypes = [C.c_void_p]
     L.mr_records.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(RecordsParams), C.c_void_p, C.c_char_p, u64p,
                              C.POINTER(C.c_void_p)]
+    L.mr_sr_names_create.argtypes = [C.c_void_p, C.c_char_p, u64p, u32p, u64p, C.c_uint32, C.POINTER(C.c_void_p)]
+    L.mr_sr_names_destroy.argtypes = [C.c_void_p]
+    L.mr_coords_records.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(CoordsParams), C.c_void_p, C.c_char_p, u64p,
+                                    C.POINTER(C.c_void_p)]
     L.mr_text_get.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), u64p]
     L.mr_text_free.argtypes = [C.c_void_p]
     _lib = L
@@ -338,11 +346,30 @@ class Context:
         printed on the device (mr_records); unitigs: Unitigs for the sequence column (-u), None for -l."""
         if result.h is None:
             raise MrError("records() needs a Result that kept its native object (align(..., keep=True) or graph())")
-        enc = [n.encode() if isinstance(n, str) else bytes(n) for n in names]
-        off = np.concatenate([[0], np.cumsum([len(n) for n in enc])]).astype(np.uint64)
+        enc, off = _joined(names)
         t = C.c_void_p()
         self.check(self.L.mr_records(self.h, result.h, C.byref(params), unitigs.h if unitigs is not None else None,
-                                     b"".join(enc), _p(off, u64p), C.byref(t)))
+                                     enc, _p(off, u64p), C.byref(t)))
+        return self._text(t)
+
+    def sr_names(self, names, path_ids, path_off):
+        """The super-reads' names (FASTA headers after '>') and unitig paths (CSR, as SuperReads.unitig_ids /
+        unitig_off) on this context's device (mr_sr_names_create), for coords_records()."""
+        return SrNames(self, names, path_ids, path_off)
+
+    def coords_records(self, result, names, compact=True, zero_match=False, *, sr_names):
+        """The jf_aligner coords lines of `result` (this context's latest, kept with keep=True, or from graph()),
+        printed on the device (mr_coords_records): compact is the tool's default format (--compact toggles it off),
+        zero_match is -0.  names: the reads' names; sr_names: an SrNames of the table the rows' `sr` indexes."""
+        if result.h is None:
+            raise MrError("coords_records() needs a Result that kept its native object (align(..., keep=True) or graph())")
+        enc, off = _joined(names)
+        p = CoordsParams(compact=int(bool(compact)), zero_match=int(bool(zero_match)))
+        t = C.c_void_p()
+        self.check(self.L.mr_coords_records(self.h, result.h, C.byref(p), sr_names.h, enc, _p(off, u64p), C.byref(t)))
+        return self._text(t)
+
+    def _text(self, t):
         try:
             p, n = C.c_void_p(), C.c_uint64()
             self.check(self.L.mr_text_get(t, C.byref(p), C.byref(n)))
@@ -441,6 +468,13 @@ class Index:
         return idx, nb
 
 
+def _joined(names):
+    """names (str or bytes) back to back, and their n + 1 offsets"""
+    enc = [n.encode() if isinstance(n, str) else bytes(n) for n in names]
+    off = np.concatenate([[0], np.cumsum([len(n) for n in enc])]).astype(np.uint64)
+    return b"".join(enc), off
+
+
 def _arr(ptr, n, dtype):
     if n == 0 or not ptr:
         return np.zeros(0, dtype=dtype)
@@ -458,6 +492,22 @@ class Unitigs:
     def close(self):
         if self.h:
             self.ctx.L.mr_unitigs_destroy(self.h)
+            self.h = None
+
+
+class SrNames:
+    def __init__(self, ctx, names, path_ids, path_off):
+        self.ctx = ctx
+        enc, off = _joined(names)
+        ids = np.ascontiguousarray(path_ids if len(path_ids) else [0], dtype=np.uint32)
+        poff = np.ascontiguousarray(path_off, dtype=np.uint64)
+        h = C.c_void_p()
+        ctx.check(ctx.L.mr_sr_names_create(ctx.h, enc, _p(off, u64p), _p(ids, u32p), _p(poff, u64p), len(off) - 1, C.byref(h)))
+        self.h = h
+
+    def close(self):
+        if self.h:
+            self.ctx.L.mr_sr_names_destroy(self.h)
             self.h = None
 
 

@@ -84,9 +84,14 @@ static int download_rows(mr_context* ctx, mr_workspace& ws, mr_result* res, cons
   return MR_OK;
 }
 
-// Stamps a finished result; with a graph, mr_records may read its rows where they are until the next batch.
-static void remember_rows(mr_workspace& ws, mr_result* res, const graph_args* GA, uint64_t S, int max_rows) {
+// Stamps a finished result: mr_coords_records may read its rows where they are until the next batch, and with a
+// graph mr_records may too.
+static void remember_rows(mr_workspace& ws, mr_result* res, const coords_soa& fin, uint32_t nreads, const graph_args* GA,
+                          uint64_t S, int max_rows) {
   res->stamp = ++ws.stamp;
+  ws.rows_stamp = res->stamp;
+  ws.last_coords = rows_args{ nreads, S, ws.read_coords.as<uint64_t>(), ws.read_len.as<uint32_t>(), fin,
+                              ws.kinfo.as<int32_t>(), ws.binfo.as<int32_t>() };
   if(!GA) return;
   ws.graph_stamp = res->stamp;
   ws.last_graph = *GA; ws.last_rows = S; ws.last_max_rows = max_rows;
@@ -1226,7 +1231,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
   cudaStream_t st = ctx->stream;
   if(!ctx->ws) ctx->ws = new mr_workspace;
   mr_workspace& ws = *ctx->ws;
-  ws.graph_stamp = 0;                       // the rows of the previous result are overwritten from here on
+  ws.graph_stamp = ws.rows_stamp = 0;      // the rows of the previous result are overwritten from here on
   const index_view& iv = idx->view;
   const uint32_t k = iv.k;
   const uint64_t T = h_read_start[nreads];
@@ -1680,7 +1685,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
   timer.end();
   MR_CUDA(ctx, ctx->wait(st));
   MR_TRACE_MSG("batch done");
-  remember_rows(ws, res.get(), graph ? &GA : nullptr, S, max_rows);
+  remember_rows(ws, res.get(), fin, nreads, graph ? &GA : nullptr, S, max_rows);
   *out = res.release();
   return MR_OK;
 }
@@ -1807,7 +1812,7 @@ int mr_graph_batch(mr_context* ctx, const mr_params* p, const mr_result_view* ro
   MR_CUDA(ctx, cudaSetDevice(ctx->device));
   if(!ctx->ws) ctx->ws = new mr_workspace;
   mr_workspace& ws = *ctx->ws;
-  ws.graph_stamp = 0;
+  ws.graph_stamp = ws.rows_stamp = 0;
   cudaStream_t st = ctx->stream;
   const uint32_t nreads = rows->nreads;
   const uint64_t S = rows->ncoords, Sc = std::max<uint64_t>(S, 1);
@@ -1872,7 +1877,7 @@ int mr_graph_batch(mr_context* ctx, const mr_params* p, const mr_result_view* ro
   timer.end();
   MR_CUDA(ctx, ctx->wait(st));
   timer.collect();
-  remember_rows(ws, res.get(), &GA, S, max_rows);
+  remember_rows(ws, res.get(), fin, nreads, &GA, S, max_rows);
   *out = res.release();
   return MR_OK;
 }

@@ -69,6 +69,16 @@ struct graph_args {
   double  *imp_s, *imp_e;
 };
 
+// The final rows of a batch where it left them on the device (mr_coords_records reads them there).
+struct rows_args {
+  uint32_t nreads;
+  uint64_t nrows;
+  const uint64_t* read_coords;
+  const uint32_t* read_len;
+  coords_soa c;
+  const int32_t *kinfo, *binfo;
+};
+
 // Scratch that lives in the context and is reused from batch to batch.
 struct mr_workspace {
   dev_buf bases, codes, nmask, read_start, read_len, tile_read, tile_pos, tile_first, tile_cand, tile_tbase;
@@ -85,9 +95,11 @@ struct mr_workspace {
   dev_buf tap_lens, tap_cf, tap_cb, group_lists, chain_pay, removed, chainW;
   dev_buf scan_scratch;
   prim::sort_scratch sort;
-  // mr_records: where the latest result's rows and graph nodes are (its stamp, 0: none with a graph), and scratch
-  uint64_t stamp = 0, graph_stamp = 0;
+  // mr_records: where the latest result's rows and graph nodes are (its stamp, 0: none with a graph), and scratch;
+  // mr_coords_records: where the latest result's rows are (rows_stamp, 0: none), for results with or without a graph
+  uint64_t stamp = 0, graph_stamp = 0, rows_stamp = 0;
   graph_args last_graph;
+  rows_args last_coords;
   uint64_t last_rows = 0;
   int last_max_rows = 0;
   dev_buf rec_cand, rec_i32, rec_f64, rec_info, rec_lines, rec_linf, rec_names, rec_text;
@@ -98,6 +110,18 @@ struct mr_workspace {
   std::vector<mr_staged*> staged_pool;      // device input buffers of staged batches, recycled (cudaMalloc synchronises the device)
   ~mr_workspace() { for(auto p : pinned_pool) delete p; for(auto p : text_pool) delete p; for(auto s : staged_pool) delete s; }
 };
+
+// text printed on the device (mr_records, mr_coords_records), in a pinned slab of the context's pool
+struct mr_text {
+  mr_context* ctx = nullptr;
+  pinned_buf* host = nullptr;
+  uint64_t size = 0;
+};
+// records.cu, shared by the two printers: the reads' names on the device (through a pinned staging buffer of the
+// workspace; *d_off: nreads + 1 offsets from 0, *d_names: the bytes), and a slab of the pool for `bytes` of text
+int upload_read_names(mr_context* ctx, mr_workspace& ws, const char* names, const uint64_t* name_off, uint32_t nreads,
+                      const uint64_t** d_off, const char** d_names);
+int take_text_slab(mr_context* ctx, mr_workspace& ws, mr_text* t, uint64_t bytes);
 
 struct mr_result {
   mr_context* ctx = nullptr;

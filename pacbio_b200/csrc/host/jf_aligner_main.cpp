@@ -112,6 +112,15 @@ int main(int argc, char* argv[]) {
       fputs(" Qname\n", out);
     }
     if(details) for(auto c : DS.ctx) mr_context_keep_taps(c, 1);
+    // The coords lines are printed on the device right after each batch (mr_coords_records); --details keeps both
+    // files on the host formatter, which needs the taps of the result there.
+    mrh::device_sr_names DN;
+    mrh::records_fn device;
+    const mr_coords_params cp = { compact ? 1 : 0, zero_match ? 1 : 0 };
+    if(!details) {
+      DN.upload(DS, SR);
+      device = [&](mr_context* c, const mr_result* r, const mrh::read_batch& b) { return mrh::device_coords(c, r, cp, DN.of(c), b.name); };
+    }
     mrh::text_buf dtext;
     mrh::run_pipeline(DS, pacbio, P,
       [&](const mr_result* r, const mr_result_view& v, const mrh::read_batch& b, std::vector<mrh::text_buf>& parts) {
@@ -122,7 +131,7 @@ int main(int argc, char* argv[]) {
           mrh::format_details(r, b, SR, dtext);
           fwrite(dtext.data(), 1, dtext.size(), details);
         }
-      }, out);
+      }, out, 0, device);
     if(out != stdout) fclose(out);
     if(details) fclose(details);
   } catch(std::exception& e) {

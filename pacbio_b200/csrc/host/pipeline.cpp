@@ -397,15 +397,55 @@ uint64_t run_pipeline(device_set& ds, const std::vector<std::string>& read_paths
   return total_bases;
 }
 
+namespace {
+// names back to back and their offsets, as the C ABI takes them
+void join_names(const std::vector<std::string>& names, std::string& all, std::vector<uint64_t>& off) {
+  off.assign(1, 0);
+  off.reserve(names.size() + 1);
+  for(const auto& n : names) { all += n; off.push_back(all.size()); }
+}
+}
+
 mr_text* device_records(mr_context* ctx, const mr_result* r, const mr_records_params& p, const mr_unitigs* u,
                         const std::vector<std::string>& names) {
   std::string all;
-  std::vector<uint64_t> off(1, 0);
-  off.reserve(names.size() + 1);
-  for(const auto& n : names) { all += n; off.push_back(all.size()); }
+  std::vector<uint64_t> off;
+  join_names(names, all, off);
   mr_text* t = nullptr;
   if(mr_records(ctx, r, &p, u, all.data(), off.data(), &t) != MR_OK) throw std::runtime_error(mr_last_error(ctx));
   return t;
+}
+
+mr_text* device_coords(mr_context* ctx, const mr_result* r, const mr_coords_params& p, const mr_sr_names* s,
+                       const std::vector<std::string>& names) {
+  std::string all;
+  std::vector<uint64_t> off;
+  join_names(names, all, off);
+  mr_text* t = nullptr;
+  if(mr_coords_records(ctx, r, &p, s, all.data(), off.data(), &t) != MR_OK) throw std::runtime_error(mr_last_error(ctx));
+  return t;
+}
+
+void device_sr_names::upload(const device_set& ds, const super_reads& SR) {
+  std::string all;
+  std::vector<uint64_t> off;
+  join_names(SR.name, all, off);
+  for(mr_context* c : ds.ctx) {
+    const int d = mr_context_device(c);
+    if(std::find(device.begin(), device.end(), d) != device.end()) continue;
+    mr_sr_names* x = nullptr;
+    if(mr_sr_names_create(c, all.data(), off.data(), SR.unitig_ids.empty() ? nullptr : SR.unitig_ids.data(), SR.unitig_off.data(),
+                          SR.nseq(), &x) != MR_OK)
+      throw std::runtime_error(std::string("mr_sr_names_create: ") + mr_last_error(c));
+    device.push_back(d);
+    s.push_back(x);
+  }
+}
+
+const mr_sr_names* device_sr_names::of(mr_context* ctx) const {
+  const int d = mr_context_device(ctx);
+  for(size_t i = 0; i < device.size(); ++i) if(device[i] == d) return s[i];
+  return nullptr;
 }
 
 void device_unitigs::upload(const device_set& ds, const unitigs& U) {

@@ -76,7 +76,7 @@ void add_streams(device_set& ds, unsigned per_device);
 // format(result, view, batch, parts): the batch's text in parts[], written by the pipeline when it returns (host
 // formatting, on the one formatter thread)
 typedef std::function<void(const mr_result*, const mr_result_view&, const read_batch&, std::vector<text_buf>&)> format_fn;
-// records(context, result, batch): the batch's text produced on the device (mr_records), called by the aligner
+// records(context, result, batch): the batch's text produced on the device (mr_records, mr_coords_records), called by the aligner
 // thread of `context` right after the batch is aligned, while its rows are still on the device.  When given, it
 // replaces `format` and the formatter thread only writes the text; it throws std::runtime_error on failure.
 typedef std::function<mr_text*(mr_context*, const mr_result*, const read_batch&)> records_fn;
@@ -98,5 +98,17 @@ struct device_unitigs {
   const mr_unitigs* of(mr_context* ctx) const;
 };
 mr_records_params records_params(const graph_options& g);
+
+// mr_coords_records over a batch of a tool: the reads' names as the C ABI takes them, errors as exceptions
+mr_text* device_coords(mr_context* ctx, const mr_result* r, const mr_coords_params& p, const mr_sr_names* s,
+                       const std::vector<std::string>& names);
+// the super-reads' names and paths on every device of ds (one upload per device, shared by its contexts)
+struct device_sr_names {
+  std::vector<int> device;
+  std::vector<mr_sr_names*> s;
+  ~device_sr_names() { for(auto x : s) mr_sr_names_destroy(x); }
+  void upload(const device_set& ds, const super_reads& SR);
+  const mr_sr_names* of(mr_context* ctx) const;
+};
 
 } // namespace mrh

@@ -326,6 +326,45 @@ int mrh_format_records(const mr_result* r, const uint32_t* path_ids, const uint6
     return -1;
   }
 }
+// The host coords formatter (mrh::format_coords, the reference of the device printer and the tool's --details path)
+// over a result: the super-reads' names and unitig paths (CSR, path_ids may be NULL when all paths are empty), the
+// reads' names and lengths (read_start: nreads + 1 offsets), --compact and -0.  *out: malloc'ed text (mrh_free).
+// Returns 0, or -1 with the message in err.
+int mrh_format_coords(const mr_result* r, const char* sr_names, const uint64_t* sr_name_off, const uint32_t* path_ids,
+                      const uint64_t* path_off, uint32_t nseq, const char* names, const uint64_t* name_off,
+                      const uint64_t* read_start, int compact, int zero_match, char** out, uint64_t* size, char* err, size_t err_cap) {
+  try {
+    mr_result_view v;
+    if(mr_result_get(r, &v) != MR_OK) throw std::runtime_error("no result");
+    mrh::super_reads sr;
+    for(uint32_t i = 0; i < nseq; ++i) sr.name.emplace_back(sr_names + sr_name_off[i], sr_name_off[i + 1] - sr_name_off[i]);
+    sr.unitig_off.assign(path_off, path_off + nseq + 1);
+    if(path_ids) sr.unitig_ids.assign(path_ids, path_ids + path_off[nseq]);
+    for(uint64_t i = 0; i < v.ncoords; ++i)
+      if(v.sr[i] >= nseq) throw std::runtime_error("a row refers to a super-read that the names do not have");
+    mrh::read_batch b;
+    b.start.assign(read_start, read_start + v.nreads + 1);
+    for(uint32_t i = 0; i < v.nreads; ++i) b.name.emplace_back(names + name_off[i], name_off[i + 1] - name_off[i]);
+    mrh::text_buf text;
+    mrh::format_coords(v, b, 0, v.nreads, sr, compact != 0, zero_match == 0, text);
+    *out = (char*)malloc(text.size() + 1);
+    if(!*out) throw std::bad_alloc();
+    if(text.size()) memcpy(*out, text.data(), text.size());
+    *size = text.size();
+    return 0;
+  } catch(std::exception& e) {
+    if(err && err_cap) { strncpy(err, e.what(), err_cap - 1); err[err_cap - 1] = 0; }
+    return -1;
+  }
+}
+// The "%g" formatter of the coords lines (records_common.hpp) and printf, side by side: both strings of x; returns
+// whether they are equal.  Each buffer holds at least mrfmt::kGeneralMax + 1 bytes.
+int mrh_general_format_pair(double x, char* mine, char* libc) {
+  const int n = mrfmt::fmt_general(mine, x);
+  mine[n] = 0;
+  snprintf(libc, mrfmt::kGeneralMax + 1, "%g", x);
+  return strcmp(mine, libc) == 0;
+}
 void mrh_free(void* p) { free(p); }
 void mrh_tool_stage_seconds(void* p, double* align_s, double* format_s) {
   tool* t = (tool*)p; *align_s = t->last_align_s; *format_s = t->last_format_s;

@@ -21,12 +21,6 @@ struct mr_unitigs {
   dev_buf seq, off;
 };
 
-struct mr_text {
-  mr_context* ctx = nullptr;
-  pinned_buf* host = nullptr;
-  uint64_t size = 0;
-};
-
 namespace {
 
 // one candidate mega-read (overlap_graph.hpp:51-63), stored at the row of its end node
@@ -535,6 +529,40 @@ __global__ void emit_lines_kernel(rec_args A, uint64_t nlines) {
 
 } // namespace
 
+// read names, through a page-locked staging buffer (the copy then needs no wait for the caller's arrays; the buffer is
+// free again because every call that uses it ends with the stream drained)
+int upload_read_names(mr_context* ctx, mr_workspace& ws, const char* names, const uint64_t* name_off, uint32_t nreads,
+                      const uint64_t** d_off, const char** d_names) {
+  const uint64_t name_bytes = name_off[nreads] - name_off[0], off_bytes = ((uint64_t)nreads + 1) * 8;
+  MR_TRY(ws.rec_names.ensure(ctx, name_bytes + off_bytes + 64));
+  if(ws.rec_names_host.cap < name_bytes + off_bytes + 64) MR_TRY(ws.rec_names_host.ensure(ctx, (name_bytes + off_bytes) * 5 / 4 + 4096));
+  uint64_t* h_off = ws.rec_names_host.as<uint64_t>();
+  for(uint32_t r = 0; r <= nreads; ++r) h_off[r] = name_off[r] - name_off[0];
+  if(name_bytes) memcpy((char*)h_off + off_bytes, names + name_off[0], name_bytes);
+  char* q = ws.rec_names.as<char>();
+  MR_CUDA(ctx, cudaMemcpyAsync(q, h_off, off_bytes + name_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  *d_off = (const uint64_t*)q; *d_names = q + off_bytes;
+  return MR_OK;
+}
+
+int take_text_slab(mr_context* ctx, mr_workspace& ws, mr_text* t, uint64_t bytes) {
+  t->size = bytes;
+  {
+    std::lock_guard<std::mutex> lock(ws.pool_mutex);
+    if(!ws.text_pool.empty()) {                     // the largest slab: the least likely to need regrowing
+      size_t best = 0;
+      for(size_t i = 1; i < ws.text_pool.size(); ++i) if(ws.text_pool[i]->cap > ws.text_pool[best]->cap) best = i;
+      t->host = ws.text_pool[best];
+      ws.text_pool.erase(ws.text_pool.begin() + best);
+    }
+  }
+  if(!t->host) t->host = new pinned_buf;
+  // a quarter more than this batch needs: batches differ in size, and a slab that is regrown costs a cudaFreeHost (which
+  // waits for the device) and a cudaMallocHost of hundreds of megabytes
+  if(t->host->cap < bytes + 1 && t->host->ensure(ctx, bytes + bytes / 4 + (1 << 20)) != MR_OK) { delete t->host; t->host = nullptr; return MR_ENOMEM; }
+  return MR_OK;
+}
+
 extern "C" {
 
 int mr_unitigs_create(mr_context* ctx, const char* seq, const uint64_t* off, uint32_t n, mr_unitigs** out) {
@@ -607,19 +635,7 @@ int mr_records(mr_context* ctx, const mr_result* res, const mr_records_params* p
     A.nlines = (uint32_t*)(q + Sc * 8 + ((size_t)nreads + 2) * 8); }
   uint64_t* d_tot = (uint64_t*)A.err + 1;        // [0] lines, [1] bytes
   A.n_lines = d_tot;
-  // read names, through a page-locked staging buffer (the copy then needs no wait for the caller's arrays; the
-  // buffer is free again because every call ends with the stream drained)
-  const uint64_t name_bytes = name_off[nreads] - name_off[0], off_bytes = ((uint64_t)nreads + 1) * 8;
-  MR_TRY(ws.rec_names.ensure(ctx, name_bytes + off_bytes + 64));
-  if(ws.rec_names_host.cap < name_bytes + off_bytes + 64) MR_TRY(ws.rec_names_host.ensure(ctx, (name_bytes + off_bytes) * 5 / 4 + 4096));
-  {
-    uint64_t* h_off = ws.rec_names_host.as<uint64_t>();
-    for(uint32_t r = 0; r <= nreads; ++r) h_off[r] = name_off[r] - name_off[0];
-    if(name_bytes) memcpy((char*)h_off + off_bytes, names + name_off[0], name_bytes);
-    char* q = ws.rec_names.as<char>();
-    MR_CUDA(ctx, cudaMemcpyAsync(q, h_off, off_bytes + name_bytes, cudaMemcpyHostToDevice, st));
-    A.name_off = (const uint64_t*)q; A.names = q + off_bytes;
-  }
+  MR_TRY(upload_read_names(ctx, ws, names, name_off, nreads, &A.name_off, &A.names));
   if(u) { A.useq = u->seq.as<char>(); A.uoff = u->off.as<uint64_t>(); A.nu = u->n; }
   MR_CUDA(ctx, cudaMemsetAsync(A.err, 0xff, 8, st));
   MR_CUDA(ctx, cudaMemsetAsync(d_tot, 0, 16, st));
@@ -645,20 +661,7 @@ int mr_records(mr_context* ctx, const mr_result* res, const mr_records_params* p
     return ctx->fail(MR_EINVAL, (h[0] & 1) ? "unitig id of a super-read name is not in the -u file"
                                            : "component root outside the read's rows");
   const uint64_t nlines = h[1], bytes = h[2];
-  t->size = bytes;
-  {
-    std::lock_guard<std::mutex> lock(ws.pool_mutex);
-    if(!ws.text_pool.empty()) {                     // the largest slab: the least likely to need regrowing
-      size_t best = 0;
-      for(size_t i = 1; i < ws.text_pool.size(); ++i) if(ws.text_pool[i]->cap > ws.text_pool[best]->cap) best = i;
-      t->host = ws.text_pool[best];
-      ws.text_pool.erase(ws.text_pool.begin() + best);
-    }
-  }
-  if(!t->host) t->host = new pinned_buf;
-  // a quarter more than this batch needs: batches differ in size, and a slab that is regrown costs a cudaFreeHost (which
-  // waits for the device) and a cudaMallocHost of hundreds of megabytes
-  if(t->host->cap < bytes + 1 && t->host->ensure(ctx, bytes + bytes / 4 + (1 << 20)) != MR_OK) { delete t->host; t->host = nullptr; return MR_ENOMEM; }
+  MR_TRY(take_text_slab(ctx, ws, t.get(), bytes));
   if(nlines) {
     MR_TRY(ws.rec_text.ensure(ctx, bytes + 1));
     A.text = ws.rec_text.as<char>();
