@@ -550,16 +550,10 @@ __global__ void __launch_bounds__(256) read_threshold_kernel(const uint64_t* __r
 __device__ __forceinline__ void emit_hit(const index_view& iv, uint32_t read, uint32_t pb_off, uint32_t sa_rank, bool minus,
                                          uint64_t slot, uint64_t* __restrict__ keys, uint64_t* __restrict__ pays,
                                          uint32_t& n_bad) {
-  uint32_t sr, off;
-  bool inside;
-  if(iv.saloc) {
-    const uint2 l = __ldg(iv.saloc + sa_rank);
-    sr = l.x; off = l.y;
-    inside = sr != 0xffffffffu;
-  } else inside = index_locate(iv, __ldg(iv.sa + sa_rank), sr, off);
-  if(inside) {
-    const int32_t soff = minus ? -(int32_t)off : (int32_t)off;
-    keys[slot] = ((uint64_t)read << 32) | (iv.sr_base + sr);
+  const uint2 l = __ldg(iv.saloc + sa_rank);
+  if(l.x != 0xffffffffu) {
+    const int32_t soff = minus ? -(int32_t)l.y : (int32_t)l.y;
+    keys[slot] = ((uint64_t)read << 32) | (iv.sr_base + l.x);
     pays[slot] = (uint64_t)pb_off | ((uint64_t)(uint32_t)soff << 32);
   } else {
     keys[slot] = ((uint64_t)read << 32) | iv.nseq_all;
@@ -1205,25 +1199,6 @@ void mr_workspace_free(mr_workspace* ws) { delete ws; }
 
 // ================================================================================================
 // host orchestration
-// L2 persistence window over the lookup tables of one index part for the kernels launched next on
-// `st` (on == false: back to normal).  The tables (prefix counts + tails, index.cuh) are what every
-// lookup reads at random; the 20 bytes per base the seed kernel streams out would otherwise keep
-// evicting them (ncu: 40 % L2 hit rate with tables of 103 MB in a 126 MB L2).
-static void l2_window(mr_context* ctx, cudaStream_t st, const mr_index* part, bool on) {
-  if(!ctx->l2_persist_bytes || !part->lut.p) return;
-  cudaStreamAttrValue v;
-  memset(&v, 0, sizeof(v));
-  if(on) {
-    const size_t bytes = std::min(part->lut_bytes, ctx->l2_window_max);
-    v.accessPolicyWindow.base_ptr = part->lut.p;
-    v.accessPolicyWindow.num_bytes = bytes;
-    v.accessPolicyWindow.hitRatio = (float)std::min(1.0, (double)ctx->l2_persist_bytes / (double)bytes);
-    v.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    v.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-  }
-  if(cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &v) != cudaSuccess) cudaGetLastError();
-}
-
 // ================================================================================================
 static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, const packed_reads& d_bases,
                             const uint64_t* d_read_start, const uint64_t* h_read_start, uint32_t nreads,
@@ -1308,7 +1283,6 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
                   : (bytes ? seed_lookup_kernel<false, false, true> : seed_lookup_kernel<false, false, false>);
     };
     for(uint32_t part = 0; part < nparts; ++part) {
-      l2_window(ctx, st, part ? idx->more[part - 1] : idx, true);
       const index_view& pv = idx->part_view(part);
       pick(nparts > 1, pv)<<<ntiles, kSeedThreads, 0, st>>>(pv, nparts == 1 ? 3u : ((part == 0 ? 1u : 0u) | (part + 1 == nparts ? 2u : 0u)),
                                                            d_bases, d_read_start, ws.tile_read.as<uint32_t>(), ws.tile_pos.as<uint32_t>(),
@@ -1316,7 +1290,6 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
                                                            ws.rec.as<uint4>() + part * rec_stride, ws.size.as<uint32_t>(), ctr + 0, ctr + 6, ctr + 9, ctr + 10);
       MR_LAUNCHED(ctx);
     }
-    l2_window(ctx, st, idx, false);
     timer.next("count threshold");
     uint32_t nbits = 32;
     if(p->max_count > 1) { nbits = 0; while((1u << nbits) < (uint32_t)p->max_count) ++nbits; }
@@ -1337,7 +1310,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
   int sr_bits = 1;
   while((1ULL << sr_bits) <= (uint64_t)iv.nseq_all) ++sr_bits;
   MR_CUDA(ctx, cudaMemcpyAsync(h_ctr, ctr, 12 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-  MR_CUDA(ctx, ctx->wait(st));
+  MR_CUDA(ctx, cudaStreamSynchronize(st));
   if(h_ctr[11]) return ctx->fail(MR_ELIMIT, "mr_align_batch: 2^32 or more hits in one 1024-base tile; use --max-count");
   const uint64_t H = h_ctr[1];
   MR_TRACE_MSG("batch: %u reads, %llu bases, %llu lookups, %llu raw hits", nreads, (unsigned long long)T, (unsigned long long)h_ctr[0], (unsigned long long)H);
@@ -1396,7 +1369,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
       MR_TRY((prim::flag_count<head_flag>(ctx, head_flag{ skeys, iv.nseq_all }, H, ws.scan_scratch, (uint64_t*)(ctr + 3))));
     }
     MR_CUDA(ctx, cudaMemcpyAsync(h_ctr, ctr, 16 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    MR_CUDA(ctx, ctx->wait(st));
+    MR_CUDA(ctx, cudaStreamSynchronize(st));
     G = h_ctr[3];
     MR_TRACE_MSG("sorted (%s); %llu groups", read_sort ? "per read" : "device-wide", (unsigned long long)G);
     const uint64_t Hvalid = H - h_ctr[2];
@@ -1466,7 +1439,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
       max_rows_kernel<<<div_up(nreads, 256), 256, 0, st>>>(ws.read_cnt.as<uint32_t>(), nreads, ctr + 12);
       MR_LAUNCHED(ctx);
       MR_CUDA(ctx, cudaMemcpyAsync(h_ctr, ctr, 13 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-      MR_CUDA(ctx, ctx->wait(st));
+      MR_CUDA(ctx, cudaStreamSynchronize(st));
       S = h_ctr[4];
       MR_TRACE_MSG("chained; %llu rows (capacity %llu)", (unsigned long long)S, (unsigned long long)cap);
       if(S <= cap) break;
@@ -1525,7 +1498,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
                                                              ws.scan_scratch, (uint64_t*)(ctr + 7))));
     MR_CUDA(ctx, cudaMemcpyAsync(ws.hit_off.as<uint64_t>() + ntiles, ctr + 7, sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
     MR_CUDA(ctx, cudaMemcpyAsync(h_ctr + 7, ctr + 7, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    MR_CUDA(ctx, ctx->wait(st));
+    MR_CUDA(ctx, cudaStreamSynchronize(st));
     const uint64_t Hf = h_ctr[7];
     MR_TRACE_MSG("fine pass: %llu windows, %llu hits inside them", (unsigned long long)S, (unsigned long long)Hf);
     if(Hf >= (1ULL << 32)) return ctx->fail(MR_ELIMIT, "mr_align_batch: too many fine-pass hits in one batch; use smaller batches");
@@ -1568,7 +1541,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
     MR_CUDA(ctx, cudaMemsetAsync(ws.read_cnt.p, 0, ((size_t)nreads + 2) * 4, st));
     MR_TRY(launch_chain(ctx, F, ws.group_lists));
     MR_CUDA(ctx, cudaMemcpyAsync(h_ctr, ctr, 6 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    MR_CUDA(ctx, ctx->wait(st));
+    MR_CUDA(ctx, cudaStreamSynchronize(st));
     if(h_ctr[4] != S) return ctx->fail(MR_ECUDA, "mr_align_batch: internal error, the fine pass lost rows");
     A = F;
     k_coords = kk;
@@ -1661,7 +1634,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
     MR_CUDA(ctx, cudaMemcpyAsync(hcf.data(), ws.tap_cf.p, H * 4, cudaMemcpyDeviceToHost, st));
     MR_CUDA(ctx, cudaMemcpyAsync(hcb.data(), ws.tap_cb.p, H * 4, cudaMemcpyDeviceToHost, st));
     if(p->max_match) MR_CUDA(ctx, cudaMemcpyAsync(hrem.data(), ws.removed.p, H, cudaMemcpyDeviceToHost, st));
-    MR_CUDA(ctx, ctx->wait(st));
+    MR_CUDA(ctx, cudaStreamSynchronize(st));
     auto kept = [&](uint64_t i) { return hrem.empty() || !hrem[i]; };
     std::vector<uint64_t> ord(G);
     for(uint64_t g = 0; g < G; ++g) ord[g] = g;
@@ -1683,7 +1656,7 @@ static int align_batch_impl(mr_context* ctx, mr_index* idx, const mr_params* p, 
     }
   }
   timer.end();
-  MR_CUDA(ctx, ctx->wait(st));
+  MR_CUDA(ctx, cudaStreamSynchronize(st));
   MR_TRACE_MSG("batch done");
   remember_rows(ws, res.get(), fin, nreads, graph ? &GA : nullptr, S, max_rows);
   *out = res.release();
@@ -1875,7 +1848,7 @@ int mr_graph_batch(mr_context* ctx, const mr_params* p, const mr_result_view* ro
   timer.next("result download");
   MR_TRY(download_rows(ctx, ws, res.get(), fin, nreads, S, info_total, &GA));
   timer.end();
-  MR_CUDA(ctx, ctx->wait(st));
+  MR_CUDA(ctx, cudaStreamSynchronize(st));
   timer.collect();
   remember_rows(ws, res.get(), fin, nreads, &GA, S, max_rows);
   *out = res.release();

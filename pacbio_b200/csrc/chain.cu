@@ -853,112 +853,6 @@ __global__ void __launch_bounds__(128) finish_tile_kernel(chain_args A, const ui
   }
 }
 
-// The same job with FOUR lanes per chain, one for each of the running means the online least squares keeps (EX, EY,
-// EXX, EXY: four independent recurrences, each five dependent FP64 operations per hit): 21 FP64 instructions per hit
-// on the critical path instead of 41, eight chains per warp, no shared memory.  An experiment kept behind
-// MR_FINISH_QUAD=1: it shortens a lone chain but costs twice the FP64 issue slots per chain, and the phase as a whole
-// is bound by those (see launch_chain).  Lane 0 of a quad also owns VX and the super-read counters, lane 1 CXY
-// and the read counters, lane 3 NB; the products that mix two recurrences (dX ndY, dXY ndX, dXX ndY) travel by
-// shuffle.  Every quantity sees exactly the operations, in the order, of coords_acc::add.
-__global__ void __launch_bounds__(128) finish_quad_kernel(chain_args A, const uint32_t* __restrict__ list,
-                                                           const uint32_t* __restrict__ list_count, uint32_t hi, uint32_t lo) {
-  const unsigned lane = threadIdx.x & 31, q = lane & 3, qbase = lane & ~3u;
-  const uint32_t total = *list_count;
-  const uint32_t k = A.align_k ? A.align_k : A.iv.k;
-  const uint32_t stride = gridDim.x * 4 * 8;
-  for(uint32_t i0 = (blockIdx.x * 4 + (threadIdx.x >> 5)) * 8; i0 < total; i0 += stride) {
-    const uint32_t i = i0 + (lane >> 2);
-    uint32_t v = 0, nb = 0, g = 0;
-    uint64_t gs = 0;
-    if(i < total) {
-      g = list[i];
-      v = A.group_nb[g]; nb = v & 0x7fffffffu;
-      if(nb > hi) nb = 0;
-      gs = A.group_start[g];
-      if(A.group_start[g + 1] - gs <= lo) nb = 0;
-    }
-    const uint32_t maxnb = __reduce_max_sync(MR_FULL_MASK, nb);
-    if(maxnb == 0) continue;
-    const uint64_t* cp = A.chain_pay + gs;
-    double E = 0, acc = 0;
-    uint32_t cons = 0, cover = k;
-    int32_t prevw = 0;
-    uint64_t nxt[8];
-#pragma unroll
-    for(int e = 0; e < 8; ++e) nxt[e] = (uint32_t)e < nb ? cp[e] : 0;
-    for(uint32_t t0 = 0; t0 < maxnb; t0 += 8) {
-      uint64_t cur[8];
-#pragma unroll
-      for(int e = 0; e < 8; ++e) { cur[e] = nxt[e]; nxt[e] = t0 + 8 + e < nb ? cp[t0 + 8 + e] : 0; }
-#pragma unroll
-      for(int e = 0; e < 8; ++e) {
-        const uint32_t t = t0 + e;
-        const bool act = t < nb;
-        const int32_t pb = (int32_t)(uint32_t)cur[e], so = (int32_t)(uint32_t)(cur[e] >> 32);
-        const double x = (double)so, y = (double)pb;
-        const double xx = x * x, xy = x * y;
-        const double val = q == 0 ? x : (q == 1 ? y : (q == 2 ? xx : xy));
-        const double dn = (double)(t + 1), r = rcp_count(t + 1);
-        const double d = val - E;
-        const double En = E + div_by_count(d, dn, r);
-        const double nd = val - En;
-        const double dX = __shfl_sync(MR_FULL_MASK, d, qbase);                          // lane 1 needs dX
-        const double ndo = __shfl_sync(MR_FULL_MASK, nd, qbase + (q == 2 ? 1u : 0u));     // lane 2: ndY, lane 3: ndX
-        const double a = q == 1 ? dX : d, b = q >= 2 ? ndo : nd;
-        const double prod = a * b;                       // lane 0: dX ndX, lane 1: dX ndY, lane 2: dXX ndY, lane 3: dXY ndX
-        const double t2 = __shfl_sync(MR_FULL_MASK, prod, qbase + 2);
-        const double add = q == 3 ? prod - t2 : prod;
-        const int32_t w = q == 1 ? pb : so;
-        if(act) {
-          E = En;
-          acc += add;
-          if(t != 0) {
-            const uint32_t diff = (uint32_t)(w - prevw);
-            cons += diff == 1; cover += min(k, diff);
-          }
-          prevw = w;
-        }
-      }
-    }
-    const double VX = __shfl_sync(MR_FULL_MASK, acc, qbase), CXY = __shfl_sync(MR_FULL_MASK, acc, qbase + 1), NB = __shfl_sync(MR_FULL_MASK, acc, qbase + 3);
-    const double EX = __shfl_sync(MR_FULL_MASK, E, qbase), EY = __shfl_sync(MR_FULL_MASK, E, qbase + 1);
-    double stretch = 1.0, offset = EY - EX, avg_err = 0;
-    const bool fit = nb > 1;
-    if(fit) { stretch = CXY / VX; offset = NB / VX; }
-    if(__any_sync(MR_FULL_MASK, fit)) {                  // every lane of the quad runs the same sum
-      double err = 0;
-#pragma unroll
-      for(int e = 0; e < 8; ++e) nxt[e] = (uint32_t)e < nb ? cp[e] : 0;
-      for(uint32_t t0 = 0; t0 < maxnb; t0 += 8) {
-        uint64_t cur[8];
-#pragma unroll
-        for(int e = 0; e < 8; ++e) { cur[e] = nxt[e]; nxt[e] = t0 + 8 + e < nb ? cp[t0 + 8 + e] : 0; }
-#pragma unroll
-        for(int e = 0; e < 8; ++e) {
-          if(t0 + e < nb) {
-            const double x = (double)(int32_t)(uint32_t)(cur[e] >> 32), y = (double)(int32_t)(uint32_t)cur[e];
-            const double prod = stretch * x;
-            err += fabs(prod + offset - y);
-          }
-        }
-      }
-      if(fit) avg_err = err / (double)(long)nb;
-    }
-    const uint32_t pb_cons = __shfl_sync(MR_FULL_MASK, cons, qbase + 1), pb_cover = __shfl_sync(MR_FULL_MASK, cover, qbase + 1);
-    if(nb != 0 && q == 0) {
-      coords_acc c(k);
-      const uint64_t p0 = cp[0], p1 = cp[nb - 1];
-      c.first_pb = (int32_t)(uint32_t)p0; c.first_sr = (int32_t)(uint32_t)(p0 >> 32);
-      c.ppb = (int32_t)(uint32_t)p1; c.psr = (int32_t)(uint32_t)(p1 >> 32);
-      c.pb_cons = pb_cons; c.pb_cover = pb_cover; c.sr_cons = cons; c.sr_cover = cover;
-      c.n = (long)nb;
-      uint32_t read, sr;
-      group_identity(A, g, gs, read, sr);
-      publish_coords(A, gs, read, sr, (v >> 31) != 0, nb, c, stretch, offset, avg_err, A.group_iter ? A.group_iter[g] : 0);
-    }
-  }
-}
-
 // ... and of the very long chains: one warp per group
 __global__ void __launch_bounds__(128) finish_warp_kernel(chain_args A) {
   const unsigned lane = threadIdx.x & 31;
@@ -1154,25 +1048,18 @@ int launch_chain(mr_context* ctx, chain_args A, dev_buf& lists) {
     if(g_chain_trace) { snprintf(label, sizeof label, "strands, tier %d (<= %u hits)", c, c < kSmemTiers ? kTierCapHost[c] : 0u); CHAIN_TRACE(st, label); }
     snprintf(label, sizeof label, "finish %d", c); tl.open(label, st);
     if(c != 0) {
-      // MR_FINISH_QUAD=1: four lanes per chain instead of a thread per chain.  Measured on B200 (yeast shape): the
-      // longest tier alone 0.40 ms against 0.34, the whole phase 28.4 ms per step against 25.4 -- FP64 issue slots
-      // are the scarce resource, and the quad form spends 1.75 FP64 warp instructions per hit and chain where the
-      // thread form spends 0.8.
-      static const bool tile_finish = !(getenv("MR_FINISH_QUAD") && atoi(getenv("MR_FINISH_QUAD")) != 0);
       // The coords kernel runs on a stream of the highest priority: the chaining kernels of the other tiers are
       // persistent and fill every SM, and their blocks still waiting for a slot would otherwise be served before the
       // coords blocks of a tier that is already chained (timeline: coords of the longest tier ready at 0.16 ms, done
-      // at 1.1).  MR_FINISH_PRIORITY=0: the tier's own stream.
-      static const bool prio = !(getenv("MR_FINISH_PRIORITY") && atoi(getenv("MR_FINISH_PRIORITY")) == 0);
+      // at 1.1).
       cudaStream_t fs = st;
-      if(prio && ctx->hi[c - 1]) {
+      if(ctx->hi[c - 1]) {
         fs = ctx->hi[c - 1];
         MR_CUDA(ctx, cudaEventRecord(ctx->ev_hi[c - 1], st));
         MR_CUDA(ctx, cudaStreamWaitEvent(fs, ctx->ev_hi[c - 1], 0));
       }
       const uint32_t lo = c == kSmemTiers && A.window > 1 ? kTierCapHost[0] : 0u;
-      if(tile_finish) finish_tile_kernel<<<ctx->sm_count * 4, 128, 0, fs>>>(A, list, ctr + c, kThreadFinishLongMax, lo);
-      else            finish_quad_kernel<<<ctx->sm_count * 8, 128, 0, fs>>>(A, list, ctr + c, kThreadFinishLongMax, lo);
+      finish_tile_kernel<<<ctx->sm_count * 4, 128, 0, fs>>>(A, list, ctr + c, kThreadFinishLongMax, lo);
       MR_LAUNCHED(ctx);
       tl.close(fs);
       if(g_chain_trace) { snprintf(label, sizeof label, "finish, tier %d", c); CHAIN_TRACE(fs, label); }

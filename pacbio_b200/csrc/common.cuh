@@ -32,20 +32,6 @@ struct mr_context {
   bool         chain_tables = false;   // constant tables of chain.cu uploaded to this device
   std::vector<std::pair<std::string, double>> timers;
   int          sm_count = kNumSMs;
-  // L2 persistence (context.cu): bytes of L2 set aside for persisting lines, largest access-policy window
-  size_t       l2_persist_bytes = 0, l2_window_max = 0;
-
-  // Waiting for the stream.  The runtime's default is to spin, which costs a whole host core per rank for
-  // the length of every batch; with few cores per GPU (8 ranks on a 32-core box) that core is what the
-  // threads that tile and print the records are short of, so there the wait sleeps on an event instead
-  // (cudaEventBlockingSync: ~20 us later to wake up, five times a batch).  MR_BLOCKING_SYNC=0/1 overrides.
-  bool         blocking_sync = false;
-  cudaEvent_t  sync_ev = nullptr;
-  cudaError_t wait(cudaStream_t st) {
-    if(!blocking_sync) return cudaStreamSynchronize(st);
-    const cudaError_t e = cudaEventRecord(sync_ev, st);
-    return e != cudaSuccess ? e : cudaEventSynchronize(sync_ev);
-  }
 
   int fail(int code, const std::string& msg) { err = msg; return code; }
 };

@@ -1,10 +1,8 @@
 // Context management for the C ABI: one context == one GPU == one stream.
 #include "common.cuh"
 
-#include <cstdlib>
 #include <cstring>
 #include <memory>
-#include <thread>
 
 thread_local std::string g_mr_create_error;
 
@@ -33,39 +31,17 @@ int mr_context_create(int device, mr_context** out) {
   std::unique_ptr<mr_context> ctx(new mr_context);
   ctx->device = device;
   ctx->sm_count = prop.multiProcessorCount;
-  // L2 persistence for the lookup tables of an index (align.cu, seed lookup): the largest set-aside
-  // the device allows.  Off unless MR_L2_PERSIST=1: measured slower (the set-aside takes the L2 away
-  // from everything else: seed lookup 31.2 -> 34.2 ms, group sort 15.9 -> 17.1 ms per step).
-  {
-    const char* env = getenv("MR_L2_PERSIST");
-    if(env && atoi(env) != 0 && prop.persistingL2CacheMaxSize > 0 && prop.accessPolicyMaxWindowSize > 0) {
-      if(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)prop.persistingL2CacheMaxSize) == cudaSuccess) {
-        ctx->l2_persist_bytes = (size_t)prop.persistingL2CacheMaxSize;
-        ctx->l2_window_max = (size_t)prop.accessPolicyMaxWindowSize;
-      } else cudaGetLastError();
-    }
-  }
   e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking);
   if(e != cudaSuccess) { g_mr_create_error = cudaGetErrorString(e); return MR_ECUDA; }
   {
     int least = 0, greatest = 0;
     if(cudaDeviceGetStreamPriorityRange(&least, &greatest) != cudaSuccess) { cudaGetLastError(); greatest = 0; }
-    // MR_CHAIN_PRIORITY=1: the chaining kernels' streams above the main stream too (one step below the coords kernels)
-    const char* cp = getenv("MR_CHAIN_PRIORITY");
-    const int aux_prio = cp && atoi(cp) != 0 ? std::min(0, greatest + 1) : 0;
-    for(auto& a : ctx->aux) if(cudaStreamCreateWithPriority(&a, cudaStreamNonBlocking, aux_prio) != cudaSuccess) { cudaGetLastError(); a = nullptr; }
+    for(auto& a : ctx->aux) if(cudaStreamCreateWithPriority(&a, cudaStreamNonBlocking, 0) != cudaSuccess) { cudaGetLastError(); a = nullptr; }
     for(auto& a : ctx->hi) if(cudaStreamCreateWithPriority(&a, cudaStreamNonBlocking, greatest) != cudaSuccess) { cudaGetLastError(); a = nullptr; }
   }
   cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking);
   for(auto& v : ctx->ev) cudaEventCreateWithFlags(&v, cudaEventDisableTiming);
   for(auto& v : ctx->ev_hi) cudaEventCreateWithFlags(&v, cudaEventDisableTiming);
-  {
-    const char* env = getenv("MR_BLOCKING_SYNC");
-    const unsigned cores = std::thread::hardware_concurrency();
-    (void)cores;
-    ctx->blocking_sync = env && *env && atoi(env) != 0;          // opt-in: measured slower on 4 cores per GPU (e2e 104.5 -> 110.6 ms per step)
-    cudaEventCreateWithFlags(&ctx->sync_ev, cudaEventDisableTiming | cudaEventBlockingSync);
-  }
   *out = ctx.release();
   return MR_OK;
 }
@@ -80,7 +56,6 @@ void mr_context_destroy(mr_context* ctx) {
   for(auto& v : ctx->ev_hi) if(v) cudaEventDestroy(v);
   if(ctx->copy_stream) { cudaStreamSynchronize(ctx->copy_stream); cudaStreamDestroy(ctx->copy_stream); }
   for(auto& v : ctx->ev) if(v) cudaEventDestroy(v);
-  if(ctx->sync_ev) cudaEventDestroy(ctx->sync_ev);
   if(ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
 }

@@ -190,7 +190,7 @@ int mr_coords_records(mr_context* ctx, const mr_result* res, const mr_coords_par
   MR_TRY((prim::exclusive_scan<prim::ptr_in_u32, uint64_t>(ctx, prim::ptr_in_u32{ A.len }, nslots, (uint64_t*)A.off, ws.scan_scratch, d_total)));
   uint64_t h[2] = { ~0ULL, 0 };
   MR_CUDA(ctx, cudaMemcpyAsync(h, A.err, 16, cudaMemcpyDeviceToHost, st));
-  MR_CUDA(ctx, ctx->wait(st));
+  MR_CUDA(ctx, cudaStreamSynchronize(st));
   if(h[0] != ~0ULL)
     return ctx->fail(MR_EINVAL, "mr_coords_records: row " + std::to_string(h[0]) + " refers to a super-read that the names do not have (" +
                                 std::to_string(srn->nseq) + " super-reads)");
@@ -202,7 +202,7 @@ int mr_coords_records(mr_context* ctx, const mr_result* res, const mr_coords_par
     coords_emit_kernel<<<div_up(nslots, 256), 256, 0, st>>>(A);
     MR_LAUNCHED(ctx);
     MR_CUDA(ctx, cudaMemcpyAsync(t->host->p, A.text, bytes, cudaMemcpyDeviceToHost, st));
-    MR_CUDA(ctx, ctx->wait(st));
+    MR_CUDA(ctx, cudaStreamSynchronize(st));
   }
   *out = t.release();
   return MR_OK;

@@ -521,7 +521,7 @@ int launch_graph(mr_context* ctx, mr_workspace& ws, graph_args a, uint64_t S, in
   MR_TRY((prim::exclusive_scan<prim::ptr_in_u32, uint64_t>(ctx, prim::ptr_in_u32{ a.edge_cnt }, S + 1, a.edge_off, ws.scan_scratch, (uint64_t*)d_total)));
   uint64_t E = 0;
   MR_CUDA(ctx, cudaMemcpyAsync(&E, d_total, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-  MR_CUDA(ctx, ctx->wait(st));
+  MR_CUDA(ctx, cudaStreamSynchronize(st));
   MR_TRY(ws.edges.ensure(ctx, (E + 1) * sizeof(int4)));
   a.edges = ws.edges.as<int4>();
   if(E) {

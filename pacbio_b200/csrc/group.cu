@@ -77,28 +77,10 @@ struct gs_sm {
   static __device__ __forceinline__ uint64_t* cbar()   { return reinterpret_cast<uint64_t*>(gs_raw + L::bar_off) + 1; }   // [3]: chunk buffers of radix_pass_global
 };
 
-// lanes of the warp whose digit equals this lane's (d <= kGsRadix), by eight ballots, one per bit: the alternative to
-// match.any, which does the same in one instruction (a fifth of the kernel's stall samples sit on the instruction that
-// consumes its result, ncu on the human-size shape).
-__device__ __forceinline__ unsigned warp_peers(uint32_t d) {
-  unsigned peers = MR_FULL_MASK;
-#pragma unroll
-  for(int b = 0; b <= kGsDigit; ++b) {
-    const bool bit = (d >> b) & 1u;
-    const unsigned m = __ballot_sync(MR_FULL_MASK, bit);
-    peers &= bit ? m : ~m;
-  }
-  return peers;
-}
-// Measured on B200: match.any wins (group sort 5.8 against 7.0 ms per step on the yeast shape, 298 against 330 on the
-// human one; the ballot form also needs more registers than the 64 the kernel has).  MR_GSORT_BALLOT=1 keeps the A/B.
-static const bool g_gs_match = !(getenv("MR_GSORT_BALLOT") && atoi(getenv("MR_GSORT_BALLOT")) != 0);
-
 // rank of this lane's key among the keys of its warp's piece that have the same digit and come before it
 // (earlier rounds through cnt, lower lanes of this round through the match mask); d == kGsRadix: no key
-template<bool kMatch>
 __device__ __forceinline__ uint32_t rank_round(uint32_t d, uint32_t* cnt_w, unsigned lt) {
-  const unsigned peers = kMatch ? __match_any_sync(MR_FULL_MASK, d) : warp_peers(d);
+  const unsigned peers = __match_any_sync(MR_FULL_MASK, d);
   const unsigned before = __popc(peers & lt);
   uint32_t b = 0;
   if(d < (uint32_t)kGsRadix) b = cnt_w[d];
@@ -109,9 +91,8 @@ __device__ __forceinline__ uint32_t rank_round(uint32_t d, uint32_t* cnt_w, unsi
 }
 
 // the same on 16-bit counters (chunks of at most 4096 keys)
-template<bool kMatch>
 __device__ __forceinline__ uint32_t rank_round16(uint32_t d, uint16_t* cnt_w, unsigned lt) {
-  const unsigned peers = kMatch ? __match_any_sync(MR_FULL_MASK, d) : warp_peers(d);
+  const unsigned peers = __match_any_sync(MR_FULL_MASK, d);
   const unsigned before = __popc(peers & lt);
   uint32_t b = 0;
   if(d < (uint32_t)kGsRadix) b = cnt_w[d];
@@ -152,7 +133,7 @@ __device__ __forceinline__ void digit_prefix(uint32_t (*cnt)[kGsRadix], uint32_t
 // ---- (1): n <= capacity hits from (kin, pin) to (ko, po, head), sorted on (super-read - key_base), a number of
 // key_bits bits.  kin == ko is allowed (everything is read before anything is written).  `phase` counts the uses
 // of the CTA's mbarrier.  All threads call it; it starts and ends with the CTA in step.
-template<int kThreads, bool kMatch>
+template<int kThreads>
 __device__ void sort_range_smem(const uint64_t* kin, const uint64_t* pin, uint64_t* ko, uint64_t* po, uint8_t* head,
                                 uint32_t n, uint32_t key_base, int key_bits, uint32_t ib, uint64_t rhi, uint32_t& phase) {
   typedef gs_sm<kThreads> Sm;
@@ -184,7 +165,7 @@ __device__ void sort_range_smem(const uint64_t* kin, const uint64_t* pin, uint64
         const uint32_t pos = piece + i * 32;
         const bool valid = pos < n;
         e[i] = valid ? arr[pos] : 0u;
-        rk[i >> 1] |= rank_round<kMatch>(valid ? (e[i] >> shift) & (kGsRadix - 1) : (uint32_t)kGsRadix, Sm::cnt()[warp], lt) << (16 * (i & 1));
+        rk[i >> 1] |= rank_round(valid ? (e[i] >> shift) & (kGsRadix - 1) : (uint32_t)kGsRadix, Sm::cnt()[warp], lt) << (16 * (i & 1));
       }
     }
     __syncthreads();
@@ -218,7 +199,7 @@ __device__ void sort_range_smem(const uint64_t* kin, const uint64_t* pin, uint64
 // CTA ranks and scatters chunk c, two barriers per chunk.  `gc` numbers the chunks the CTA has staged so far: chunk
 // g uses buffer g % 3, whose mbarrier is then in phase (g / 3) & 1.  Chunks are cut at even hit indices so that every
 // bulk copy is 16-byte aligned (a slice that starts at an odd index gets one dead position in front).
-template<int kThreads, bool kMatch>
+template<int kThreads>
 __device__ void radix_pass_global(const uint64_t* sk, const uint64_t* sp, uint64_t* dk, uint64_t* dp, uint32_t n,
                                   int shift, uint32_t dmask, bool keep, uint32_t& gc) {
   typedef gs_sm<kThreads> Sm;
@@ -279,7 +260,7 @@ __device__ void radix_pass_global(const uint64_t* sk, const uint64_t* sp, uint64
       const uint64_t pos = c0 + q0 + i * 32;
       const bool valid = pos >= skew && pos < m;
       key[i] = kb[q0 + i * 32];
-      rk[i] = rank_round16<kMatch>(valid ? ((uint32_t)key[i] >> shift) & dmask : (uint32_t)kGsRadix, cnt[warp], lt);
+      rk[i] = rank_round16(valid ? ((uint32_t)key[i] >> shift) & dmask : (uint32_t)kGsRadix, cnt[warp], lt);
     }
     __syncthreads();
     if(threadIdx.x == 0 && c + 2 < nchunks) issue(c + 2);                // its buffer was last read while chunk c - 1 was scattered
@@ -308,7 +289,7 @@ __device__ void radix_pass_global(const uint64_t* sk, const uint64_t* sp, uint64
 
 // ---- (3): (ak, ap)[0, n) sorted on key bits [0, bits) by LSD passes; the result is left in (ak, ap) when
 // `stay`, else in (bk, bp) (the pass count is made even or odd accordingly); then the head bytes
-template<int kThreads, bool kMatch>
+template<int kThreads>
 __device__ void sort_range_global(uint64_t* ak, uint64_t* ap, uint64_t* bk, uint64_t* bp, uint8_t* head,
                                   uint32_t n, int bits, bool stay, uint32_t& gc) {
   int passes = (bits + kGsDigit - 1) / kGsDigit;
@@ -316,7 +297,7 @@ __device__ void sort_range_global(uint64_t* ak, uint64_t* ap, uint64_t* bk, uint
   if(passes) {
     const int width = max(1, (bits + passes - 1) / passes);
     for(int p = 0; p < passes; ++p) {
-      radix_pass_global<kThreads, kMatch>(ak, ap, bk, bp, n, p * width, (1u << width) - 1, false, gc);
+      radix_pass_global<kThreads>(ak, ap, bk, bp, n, p * width, (1u << width) - 1, false, gc);
       uint64_t* t = ak; ak = bk; bk = t;
       t = ap; ap = bp; bp = t;
     }
@@ -326,7 +307,7 @@ __device__ void sort_range_global(uint64_t* ak, uint64_t* ap, uint64_t* bk, uint
   __syncthreads();
 }
 
-template<int kThreads, bool kMatch>
+template<int kThreads>
 __global__ void __launch_bounds__(kThreads, kThreads == 1024 ? 1 : 2) group_sort_kernel(group_sort_args A) {
   typedef gs_sm<kThreads> Sm;
 
@@ -343,14 +324,14 @@ __global__ void __launch_bounds__(kThreads, kThreads == 1024 ? 1 : 2) group_sort
   uint8_t* head = A.head + seg;
 
   if(n <= A.cap) {
-    sort_range_smem<kThreads, kMatch>(kin, pin, ko, po, head, n, 0u, A.sr_bits, A.idx_bits, rhi, phase);
+    sort_range_smem<kThreads>(kin, pin, ko, po, head, n, 0u, A.sr_bits, A.idx_bits, rhi, phase);
   } else {
     const int low_bits = A.sr_bits > kGsDigit ? A.sr_bits - kGsDigit : 0;
     if(low_bits + (int)A.range_idx_bits > 32) {
-      sort_range_global<kThreads, kMatch>(kin, pin, ko, po, head, n, A.sr_bits, false, gc);
+      sort_range_global<kThreads>(kin, pin, ko, po, head, n, A.sr_bits, false, gc);
     } else {
       // (2): cut by the top digit, then sort runs of consecutive buckets in shared memory
-      radix_pass_global<kThreads, kMatch>(kin, pin, ko, po, n, low_bits, kGsRadix - 1, true, gc);
+      radix_pass_global<kThreads>(kin, pin, ko, po, n, low_bits, kGsRadix - 1, true, gc);
       asm volatile("fence.proxy.async;" ::: "memory");        // the bulk copies below read what this CTA just stored
       __syncthreads();
       const uint32_t rcap = A.range_cap;
@@ -360,7 +341,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == 1024 ? 1 : 2) group_sort
         if(sz == 0) { ++b; continue; }
         const uint32_t at = Sm::bstart()[b];
         if(sz > rcap) {                                       // (3) on the bucket's low bits, back into place
-          sort_range_global<kThreads, kMatch>(ko + at, po + at, kin + at, pin + at, head + at, sz, low_bits, true, gc);
+          sort_range_global<kThreads>(ko + at, po + at, kin + at, pin + at, head + at, sz, low_bits, true, gc);
           asm volatile("fence.proxy.async;" ::: "memory");
           __syncthreads();
           ++b;
@@ -376,7 +357,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == 1024 ? 1 : 2) group_sort
         }
         const uint32_t nb = b1 - b;
         const int kb = low_bits + (nb > 1 ? 32 - __clz(nb - 1) : 0);
-        sort_range_smem<kThreads, kMatch>(ko + at, po + at, ko + at, po + at, head + at, total, b << low_bits, kb, A.range_idx_bits, rhi, phase);
+        sort_range_smem<kThreads>(ko + at, po + at, ko + at, po + at, head + at, total, b << low_bits, kb, A.range_idx_bits, rhi, phase);
         b = b1;
       }
     }
@@ -413,8 +394,7 @@ int launch_group_sort(mr_context* ctx, group_sort_args A, uint32_t nreads) {
   A.cap = A.sr_bits + 5 <= 32 ? 1u << A.idx_bits : 0u;        // whole reads in shared memory: up to this many hits
   typedef void (*kernel_t)(group_sort_args);
   const bool wide = group_sort_threads() == 1024;
-  const kernel_t fn = wide ? (g_gs_match ? group_sort_kernel<1024, true> : group_sort_kernel<1024, false>)
-                           : (g_gs_match ? group_sort_kernel<512, true> : group_sort_kernel<512, false>);
+  const kernel_t fn = wide ? group_sort_kernel<1024> : group_sort_kernel<512>;
   const size_t smem = wide ? gs_layout<1024>::bytes : gs_layout<512>::bytes;
   MR_CUDA(ctx, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   fn<<<nreads, wide ? 1024 : 512, smem, ctx->stream>>>(A);

@@ -83,11 +83,6 @@ unsigned streams_per_device() {
   return 2;
 }
 
-bool stage_batches() {
-  const char* e = getenv("MR_STAGE");
-  return e && *e && *e != '0';
-}
-
 void add_streams(device_set& ds, unsigned per_device) {
   const size_t ndev = ds.ctx.size();
   for(unsigned s = 1; s < per_device; ++s) {
@@ -263,9 +258,9 @@ uint64_t run_pipeline(device_set& ds, const std::vector<std::string>& read_paths
     to_align.close();
   });
 
-  // per context: an uploader thread stages the next batch (host -> device copy on the context's copy
-  // stream, mr_stage_batch) while the aligner thread runs the kernels of the current one
-  struct staged_job { job j; mr_staged* staged; int slot = -1; };
+  // per context: an uploader thread packs the next batch into a staging slot while the aligner thread runs the
+  // kernels of the current one
+  struct staged_job { job j; int slot = -1; };
   std::vector<std::unique_ptr<bounded_queue<staged_job>>> staged;
   for(size_t g = 0; g < ds.ctx.size(); ++g) staged.emplace_back(new bounded_queue<staged_job>(1));
   std::vector<std::thread> aligners, uploaders;
@@ -275,16 +270,13 @@ uint64_t run_pipeline(device_set& ds, const std::vector<std::string>& read_paths
       job j;
       while(to_align.pop(j)) {
         staged_job sj;
-        sj.staged = nullptr;
         const uint64_t t0 = now_us();
         if(!j.batch->packed()) j.batch->pack();  // 2 bits per base + non-ACGT mask: what crosses PCIe
-        if(use_slots && !stage_batches()) {
+        if(use_slots) {
           int k = -1;
           if(free_slots[g]->pop(k) && !slot_fill(g, slots[g][k], *j.batch)) { free_slots[g]->push(std::move(k)); k = -1; }
           sj.slot = k;
         }
-        if(stage_batches() && !failed && mr_stage_batch_packed(ds.ctx[g], j.batch->codes.data(), j.batch->nmask.data(), j.batch->start.data(), j.batch->nreads(), &sj.staged) != MR_OK)
-          sj.staged = nullptr;                  // the aligner retries through mr_align_batch and reports what is wrong
         busy_upload_us += now_us() - t0;
         sj.j = std::move(j);
         staged[g]->push(std::move(sj));
@@ -295,7 +287,7 @@ uint64_t run_pipeline(device_set& ds, const std::vector<std::string>& read_paths
       staged_job sj;
       while(staged[g]->pop(sj)) {
         job j = std::move(sj.j);
-        if(failed) { if(sj.staged) mr_staged_free(sj.staged); if(sj.slot >= 0) { int k = sj.slot; free_slots[g]->push(std::move(k)); } continue; }
+        if(failed) { if(sj.slot >= 0) { int k = sj.slot; free_slots[g]->push(std::move(k)); } continue; }
         // A batch whose hits exceed a device limit (very repeat-rich reads) or the free memory is cut
         // in halves and retried; the halves are formatted in order, so the output does not change.
         std::deque<std::unique_ptr<read_batch>> work;
@@ -305,15 +297,11 @@ uint64_t run_pipeline(device_set& ds, const std::vector<std::string>& read_paths
           std::unique_ptr<read_batch> b = std::move(work.front());
           work.pop_front();
           part pt;
-          int rc;
-          if(sj.staged) { rc = mr_align_staged(ds.ctx[g], ds.idx[g], &params, sj.staged, &pt.result); sj.staged = nullptr; }
-          else {
-            if(!b->packed()) b->pack();         // a half of a batch that had to be split
-            const bool from_slot = sj.slot >= 0;
-            rc = mr_align_batch_packed(ds.ctx[g], ds.idx[g], &params, from_slot ? slots[g][sj.slot].codes : b->codes.data(),
-                                       from_slot ? slots[g][sj.slot].nmask : b->nmask.data(), b->start.data(), b->nreads(), &pt.result);
-            if(from_slot) { int k = sj.slot; sj.slot = -1; free_slots[g]->push(std::move(k)); }    // (a batch that is split is retried from its own arrays)
-          }
+          if(!b->packed()) b->pack();           // a half of a batch that had to be split
+          const bool from_slot = sj.slot >= 0;
+          const int rc = mr_align_batch_packed(ds.ctx[g], ds.idx[g], &params, from_slot ? slots[g][sj.slot].codes : b->codes.data(),
+                                               from_slot ? slots[g][sj.slot].nmask : b->nmask.data(), b->start.data(), b->nreads(), &pt.result);
+          if(from_slot) { int k = sj.slot; sj.slot = -1; free_slots[g]->push(std::move(k)); }    // (a batch that is split is retried from its own arrays)
           if(rc == MR_OK) {
             if(records) {                       // printed on the device while the rows are still there
               try { pt.text = records(ds.ctx[g], pt.result, *b); } catch(std::exception& e) { fail(e.what()); }

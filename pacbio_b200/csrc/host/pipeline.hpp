@@ -67,9 +67,6 @@ void build_indexes(device_set& ds, const std::vector<int>& devices, const super_
 // second stream because its aligner thread took a core from the threads that tile and print the records;
 // that stage costs half as much now (exact integer formatter, sequence arena).
 unsigned streams_per_device();
-// MR_STAGE=1: copy the next batch to the device while the current one is aligned (mr_stage_batch /
-// mr_align_staged); off by default until it has run on the target box
-bool stage_batches();
 // adds per_device - 1 more contexts for every device of ds, sharing the device's index
 void add_streams(device_set& ds, unsigned per_device);
 

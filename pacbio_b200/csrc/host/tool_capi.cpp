@@ -165,13 +165,9 @@ int64_t mrh_tool_run_range(void* p, unsigned threads, const char* out_path, uint
   });
   std::atomic<size_t> next(0);
   std::vector<double> busy(t->DS.ctx.size(), 0.0);
-  std::vector<std::thread> aligners, uploaders;
-  struct staged_item { size_t i; mr_staged* s; };
-  std::vector<std::unique_ptr<mrh::bounded_queue<staged_item>>> staged;
-  for(size_t s = 0; s < t->DS.ctx.size(); ++s) staged.emplace_back(new mrh::bounded_queue<staged_item>(1));
+  std::vector<std::thread> aligners;
   for(size_t s = 0; s < t->DS.ctx.size(); ++s) {
-    // the copy of a context's next batch runs (on its copy stream) while its current batch is aligned
-    uploaders.emplace_back([&, s]() {
+    aligners.emplace_back([&, s]() {
       while(true) {
         const size_t i = next++;
         if(i >= nb) break;
@@ -180,26 +176,10 @@ int64_t mrh_tool_run_range(void* p, unsigned threads, const char* out_path, uint
           cv.wait(l, [&] { return i < formatted + 3 + t->DS.ctx.size() || stop; });
           if(stop) break;
         }
-        mrh::read_batch* b = t->batches[first + i].get();
-        mr_staged* st = nullptr;
-        if(mrh::stage_batches() && mr_stage_batch_packed(t->DS.ctx[s], b->codes.data(), b->nmask.data(), b->start.data(), b->nreads(), &st) != MR_OK) {
-          std::lock_guard<std::mutex> l(m);
-          if(align_error.empty()) align_error = mr_last_error(t->DS.ctx[s]);
-          stop = true; cv.notify_all();
-          break;
-        }
-        staged[s]->push(staged_item{ i, st });
-      }
-      staged[s]->close();
-    });
-    aligners.emplace_back([&, s]() {
-      staged_item it;
-      while(staged[s]->pop(it)) {
         mr_result* r = nullptr;
         const auto a0 = std::chrono::steady_clock::now();
-        mrh::read_batch* b = t->batches[first + it.i].get();
-        const int rc = it.s ? mr_align_staged(t->DS.ctx[s], t->DS.idx[s], &t->P, it.s, &r)
-                            : mr_align_batch_packed(t->DS.ctx[s], t->DS.idx[s], &t->P, b->codes.data(), b->nmask.data(), b->start.data(), b->nreads(), &r);
+        mrh::read_batch* b = t->batches[first + i].get();
+        const int rc = mr_align_batch_packed(t->DS.ctx[s], t->DS.idx[s], &t->P, b->codes.data(), b->nmask.data(), b->start.data(), b->nreads(), &r);
         mr_text* text = nullptr;
         std::string rec_error;
         if(rc == MR_OK) {
@@ -210,14 +190,13 @@ int64_t mrh_tool_run_range(void* p, unsigned threads, const char* out_path, uint
         std::lock_guard<std::mutex> l(m);
         if(rc != MR_OK || !rec_error.empty()) {
           if(align_error.empty()) align_error = rc != MR_OK ? mr_last_error(t->DS.ctx[s]) : rec_error;
-          stop = true; cv.notify_all(); continue;
+          stop = true; cv.notify_all(); break;
         }
-        done[it.i] = r; texts[it.i] = text; ready[it.i] = 1;
+        done[i] = r; texts[i] = text; ready[i] = 1;
         cv.notify_all();
       }
     });
   }
-  for(auto& th : uploaders) th.join();
   for(auto& th : aligners) th.join();
   formatter.join();
   for(double b : busy) t->last_align_s = std::max(t->last_align_s, b);

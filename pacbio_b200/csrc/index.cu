@@ -323,25 +323,16 @@ int build_slots(mr_index* idx) {
     v.blkx = idx->blkx.as<uint4>();
   }
   v.saloc = nullptr;
-  {
-    // MR_SALOC=0: hits are located at expansion time through the block table, as before (A/B, and 8 bytes per
-    // text base less device memory)
-    const char* knob = getenv("MR_SALOC");
-    if(!(knob && atoi(knob) == 0)) {
-      MR_TRY(idx->saloc.ensure(ctx, (size_t)v.nsa * sizeof(uint2)));
-      saloc_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(v, idx->saloc.as<uint2>());
-      MR_LAUNCHED(ctx);
-      MR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-      v.saloc = idx->saloc.as<uint2>();
-    }
-  }
+  MR_TRY(idx->saloc.ensure(ctx, (size_t)v.nsa * sizeof(uint2)));
+  saloc_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(v, idx->saloc.as<uint2>());
+  MR_LAUNCHED(ctx);
+  MR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  v.saloc = idx->saloc.as<uint2>();
   v.nib = nullptr; v.gbase = nullptr;
   // The nibble form of the prefix counts pays while most groups of 64 buckets hold no bucket of 15 entries:
-  // a mean bucket of up to ~4 (the yeast-size index: 2.1).  MR_NIB=0 switches it off (A/B), MR_NIB=1 forces it.
+  // a mean bucket of up to ~4 (the yeast-size index: 2.1).
   const uint32_t nprefix = 1u << (2 * v.mi);
-  const char* knob = getenv("MR_NIB");
-  const bool forced = knob && atoi(knob) == 1, off = knob && atoi(knob) == 0;
-  if(off || v.mi < 3 || (!forced && (uint64_t)v.nsa > (uint64_t)nprefix * 4)) return MR_OK;
+  if(v.mi < 3 || (uint64_t)v.nsa > (uint64_t)nprefix * 4) return MR_OK;
   const uint32_t ngroups = nprefix / 32;
   MR_TRY(idx->nib.ensure(ctx, (size_t)ngroups * sizeof(ulonglong2)));
   MR_TRY(idx->gbase.ensure(ctx, (size_t)ngroups * sizeof(uint32_t)));
@@ -354,7 +345,7 @@ int build_slots(mr_index* idx) {
   unsigned long long n_overflow = 0;
   MR_CUDA(ctx, cudaMemcpyAsync(&n_overflow, ovf.p, sizeof n_overflow, cudaMemcpyDeviceToHost, ctx->stream));
   MR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if(!forced && n_overflow * 4 > ngroups) { idx->nib.release(); idx->gbase.release(); return MR_OK; }    // too many groups fall back: not worth the extra read
+  if(n_overflow * 4 > ngroups) { idx->nib.release(); idx->gbase.release(); return MR_OK; }    // too many groups fall back: not worth the extra read
   v.nib = idx->nib.as<ulonglong2>(); v.gbase = idx->gbase.as<uint32_t>();
   idx->nib_overflow_groups = n_overflow;
   return MR_OK;

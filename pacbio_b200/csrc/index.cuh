@@ -80,8 +80,7 @@ struct mr_index {
   dev_buf  nib, gbase;               // see index_view::nib (derived; not in index files)
   dev_buf  saloc;                    // see index_view::saloc (derived; not in index files)
   dev_buf  blkx;                     // uint4[(n>>8)+1]: see index_view::blkx (derived; not in index files)
-  dev_buf  lut;                      // counts and tails live side by side in this one allocation, so that
-                                     // a single L2 access-policy window covers what a lookup reads
+  dev_buf  lut;                      // counts and tails live side by side in this one allocation
   int alloc_lut(mr_context* c, size_t counts_bytes, size_t tails_bytes) {
     const size_t off = (counts_bytes + 255) & ~(size_t)255;
     const int rc = lut.ensure(c, off + tails_bytes);
@@ -106,40 +105,16 @@ struct mr_index {
   ~mr_index() { for(mr_index* m_ : more) delete m_; }
 };
 
-// L2 eviction-priority hint for the loads of the lookup tables (kHint): the seed kernel streams
-// 20 bytes per read base through the L2 next to its random reads of tables that would just fit it;
-// loads tagged evict_last keep the tables' lines in preference to the streamed ones.
-__device__ __forceinline__ uint64_t l2_evict_last_policy() {
-  uint64_t p;
-  asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-template<bool kHint>
-__device__ __forceinline__ uint4 table_load_v4(const uint4* ptr, uint64_t pol) {
-  if(!kHint) return __ldg(ptr);
-  uint4 v;
-  asm("ld.global.nc.L2::cache_hint.v4.u32 {%0, %1, %2, %3}, [%4], %5;" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(ptr), "l"(pol));
-  return v;
-}
-template<bool kHint>
-__device__ __forceinline__ uint32_t table_load_u32(const uint32_t* ptr, uint64_t pol) {
-  if(!kHint) return __ldg(ptr);
-  uint32_t v;
-  asm("ld.global.nc.L2::cache_hint.u32 %0, [%1], %2;" : "=r"(v) : "l"(ptr), "l"(pol));
-  return v;
-}
-
 // counts[p], counts[p + 1] with one 16-byte load (plus a 4-byte one when p % 4 == 3): the two
 // entries almost always share a 32-byte sector, and a random sector fetched once must not be
 // requested a second time by a separate load instruction after it has left the L1.
-template<bool kHint = false>
-__device__ __forceinline__ void load_count_pair(const uint32_t* __restrict__ counts, uint32_t p, uint32_t& c0, uint32_t& c1, uint64_t pol = 0) {
-  const uint4 v = table_load_v4<kHint>(reinterpret_cast<const uint4*>(counts) + (p >> 2), pol);
+__device__ __forceinline__ void load_count_pair(const uint32_t* __restrict__ counts, uint32_t p, uint32_t& c0, uint32_t& c1) {
+  const uint4 v = __ldg(reinterpret_cast<const uint4*>(counts) + (p >> 2));
   switch(p & 3) {
   case 0: c0 = v.x; c1 = v.y; break;
   case 1: c0 = v.y; c1 = v.z; break;
   case 2: c0 = v.z; c1 = v.w; break;
-  default: c0 = v.w; c1 = table_load_u32<kHint>(counts + p + 1, pol);
+  default: c0 = v.w; c1 = __ldg(counts + p + 1);
   }
 }
 
@@ -149,8 +124,8 @@ __device__ __forceinline__ uint32_t nibble_sum(uint64_t x) {
   return (uint32_t)((t * 0x0101010101010101ULL) >> 56);
 }
 // bounds [c0, c1) of the bucket of prefix p: from the nibble record when the index has one (kNib), else counts[p], counts[p + 1]
-template<bool kNib, bool kHint = false>
-__device__ __forceinline__ void bucket_bounds(const index_view& iv, uint32_t p, uint32_t& c0, uint32_t& c1, uint64_t pol = 0) {
+template<bool kNib>
+__device__ __forceinline__ void bucket_bounds(const index_view& iv, uint32_t p, uint32_t& c0, uint32_t& c1) {
   if(kNib) {
     const uint32_t g = p >> 5, j = p & 31;
     const ulonglong2 rec = __ldg(iv.nib + g);
@@ -164,18 +139,10 @@ __device__ __forceinline__ void bucket_bounds(const index_view& iv, uint32_t p, 
       return;
     }
   }
-  load_count_pair<kHint>(iv.counts, p, c0, c1, pol);
+  load_count_pair(iv.counts, p, c0, c1);
 }
 
-template<bool kHint = false>
-__device__ __forceinline__ uint32_t tail_word(const index_view& iv, uint32_t word_index, uint64_t pol = 0);
-template<bool kHint = false>
-__device__ __forceinline__ uint32_t load_tail(const index_view& iv, uint32_t i, uint64_t pol = 0) {
-  if(kHint) {                                    // through the aligned word that holds the entry
-    if(iv.tail_bytes == 1) return (tail_word<true>(iv, i >> 2, pol) >> (8 * (i & 3))) & 0xffu;
-    if(iv.tail_bytes == 2) return (tail_word<true>(iv, i >> 1, pol) >> (16 * (i & 1))) & 0xffffu;
-    return tail_word<true>(iv, i, pol);
-  }
+__device__ __forceinline__ uint32_t load_tail(const index_view& iv, uint32_t i) {
   if(iv.tail_bytes == 1) return __ldg(reinterpret_cast<const uint8_t*>(iv.tails) + i);
   if(iv.tail_bytes == 2) return __ldg(reinterpret_cast<const uint16_t*>(iv.tails) + i);
   return __ldg(reinterpret_cast<const uint32_t*>(iv.tails) + i);
@@ -185,22 +152,20 @@ __device__ __forceinline__ uint32_t load_tail(const index_view& iv, uint32_t i, 
 // tails are read as aligned 32-bit words (4 / 2 / 1 entries each) and compared with the per-byte /
 // per-halfword SIMD instructions: a bucket of 8 one-byte tails costs 2-3 loads and ~25 instructions
 // instead of 8 loads and ~80.
-template<bool kHint>
-__device__ __forceinline__ uint32_t tail_word(const index_view& iv, uint32_t word_index, uint64_t pol) {
-  return table_load_u32<kHint>(reinterpret_cast<const uint32_t*>(iv.tails) + word_index, pol);
+__device__ __forceinline__ uint32_t tail_word(const index_view& iv, uint32_t word_index) {
+  return __ldg(reinterpret_cast<const uint32_t*>(iv.tails) + word_index);
 }
 __device__ __forceinline__ uint32_t tail_word_of(const index_view& iv, uint32_t entry) {   // word holding `entry`
   return iv.tail_bytes == 1 ? entry >> 2 : (iv.tail_bytes == 2 ? entry >> 1 : entry);
 }
 
 // entries of tails[a0, a1) that are < t (less) and <= t (leq); w0 = the word holding entry a0, already loaded
-template<bool kHint = false>
 __device__ __forceinline__ void bucket_count(const index_view& iv, uint32_t a0, uint32_t a1, uint32_t t, uint32_t w0,
-                                             uint32_t& less, uint32_t& leq, uint64_t pol = 0) {
+                                             uint32_t& less, uint32_t& leq) {
   less = 0; leq = 0;
   if(iv.tail_bytes == 4) {
     less = w0 < t; leq = w0 <= t;
-    for(uint32_t i = a0 + 1; i < a1; ++i) { const uint32_t v = tail_word<kHint>(iv, i, pol); less += v < t; leq += v <= t; }
+    for(uint32_t i = a0 + 1; i < a1; ++i) { const uint32_t v = tail_word(iv, i); less += v < t; leq += v <= t; }
     return;
   }
   const bool bytes = iv.tail_bytes == 1;
@@ -208,7 +173,7 @@ __device__ __forceinline__ void bucket_count(const index_view& iv, uint32_t a0, 
   const uint32_t trep = bytes ? t * 0x01010101u : t * 0x00010001u;
   uint32_t w = w0;
   for(uint32_t base = a0 & ~((1u << epw_shift) - 1); base < a1; base += 1u << epw_shift) {
-    if(base > a0) w = tail_word<kHint>(iv, base >> epw_shift, pol);
+    if(base > a0) w = tail_word(iv, base >> epw_shift);
     const uint32_t skip = base < a0 ? a0 - base : 0;                         // entries of this word before the bucket
     const uint32_t have = min(1u << epw_shift, a1 - base);                   // entries of this word inside [.., a1)
     const uint32_t hi = have == (1u << epw_shift) ? 0xffffffffu : ((1u << (ebits * have)) - 1);
@@ -221,18 +186,17 @@ __device__ __forceinline__ void bucket_count(const index_view& iv, uint32_t a0, 
 }
 
 // [lo, hi) of tails[a0, a1) equal to t
-template<bool kHint = false>
 __device__ __forceinline__ void bucket_range(const index_view& iv, uint32_t a0, uint32_t a1, uint32_t t, uint32_t w0,
-                                             uint32_t& lo, uint32_t& hi, uint64_t pol = 0) {
+                                             uint32_t& lo, uint32_t& hi) {
   if(a1 - a0 <= 64) {
     uint32_t less, leq;
-    bucket_count<kHint>(iv, a0, a1, t, w0, less, leq, pol);
+    bucket_count(iv, a0, a1, t, w0, less, leq);
     lo = a0 + less; hi = a0 + leq;
   } else {
     uint32_t a = a0, b = a1;
-    while(a < b) { const uint32_t mid = a + ((b - a) >> 1); if(load_tail<kHint>(iv, mid, pol) < t) a = mid + 1; else b = mid; }
+    while(a < b) { const uint32_t mid = a + ((b - a) >> 1); if(load_tail(iv, mid) < t) a = mid + 1; else b = mid; }
     lo = a; b = a1;
-    while(a < b) { const uint32_t mid = a + ((b - a) >> 1); if(load_tail<kHint>(iv, mid, pol) <= t) a = mid + 1; else b = mid; }
+    while(a < b) { const uint32_t mid = a + ((b - a) >> 1); if(load_tail(iv, mid) <= t) a = mid + 1; else b = mid; }
     hi = a;
   }
 }
@@ -240,7 +204,7 @@ __device__ __forceinline__ void bucket_range(const index_view& iv, uint32_t a0, 
 // bucket_range for one-byte tails (k - mi <= 4: the production mer lengths), without the width dispatch
 __device__ __forceinline__ void bucket_range_bytes(const index_view& iv, uint32_t a0, uint32_t a1, uint32_t t, uint32_t w0,
                                                    uint32_t& lo, uint32_t& hi) {
-  if(a1 - a0 > 64) { bucket_range<false>(iv, a0, a1, t, w0, lo, hi); return; }
+  if(a1 - a0 > 64) { bucket_range(iv, a0, a1, t, w0, lo, hi); return; }
   const uint32_t trep = t * 0x01010101u;
   const uint32_t* words = reinterpret_cast<const uint32_t*>(iv.tails);
   uint32_t less = 0, leq = 0, w = w0;

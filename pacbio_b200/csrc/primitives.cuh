@@ -228,22 +228,23 @@ __global__ void __launch_bounds__(kSortThreads) radix_hist_kernel(const K* __res
   if(threadIdx.x < kRadix) table[(uint64_t)threadIdx.x * nblocks + blockIdx.x] = h[threadIdx.x];   // digit-major
 }
 
-// Each warp owns a contiguous 512-key slice of the tile and walks it 32 keys at a time, so the
+// Each warp owns a contiguous 256-key slice of the tile and walks it 32 keys at a time, so the
 // rank of a key among equal digits is (earlier warps) + (earlier rounds of this warp) + (lower
 // lanes of this round): order preserving, hence stable.
-// kThreads threads rank a tile of kSortTile keys, kSortTile / kThreads each.  256 threads x 16 keys keeps 16 keys and
-// ranks per thread in registers and leaves the SM at ~22 % occupancy with every warp waiting on its loads
-// (ncu: long_scoreboard); 512 x 8 halves the registers and doubles the warps in flight.
-template<typename K, typename V, int kBits, int kThreads>
-__global__ void __launch_bounds__(kThreads) radix_scatter_kernel(const K* __restrict__ kin, const V* __restrict__ vin,
+// kScatterThreads threads rank a tile of kSortTile keys, 8 each.  256 threads x 16 keys keeps 16 keys and ranks per
+// thread in registers and leaves the SM at ~22 % occupancy with every warp waiting on its loads (ncu:
+// long_scoreboard); 512 x 8 halves the registers and doubles the warps in flight.
+constexpr int kScatterThreads = 512;
+template<typename K, typename V, int kBits>
+__global__ void __launch_bounds__(kScatterThreads) radix_scatter_kernel(const K* __restrict__ kin, const V* __restrict__ vin,
                                                                   K* __restrict__ kout, V* __restrict__ vout,
                                                                   uint64_t n, int shift,
                                                                   const uint64_t* __restrict__ offsets, uint32_t nblocks) {
-  constexpr int kRadix = 1 << kBits, kWarps = kThreads / 32, kItems = kSortTile / kThreads;
+  constexpr int kRadix = 1 << kBits, kWarps = kScatterThreads / 32, kItems = kSortTile / kScatterThreads;
   __shared__ uint32_t cnt[kWarps][kRadix];
   __shared__ uint32_t wrel[kWarps][kRadix];       // first slot of warp w's keys with digit d, relative to dbase[d]
   __shared__ uint64_t dbase[kRadix];              // first slot of this tile's keys with digit d
-  for(int i = threadIdx.x; i < kWarps * kRadix; i += kThreads) (&cnt[0][0])[i] = 0;
+  for(int i = threadIdx.x; i < kWarps * kRadix; i += kScatterThreads) (&cnt[0][0])[i] = 0;
   __syncthreads();
   const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const uint64_t base = (uint64_t)blockIdx.x * kSortTile + (uint64_t)warp * (32 * kItems);
@@ -265,7 +266,7 @@ __global__ void __launch_bounds__(kThreads) radix_scatter_kernel(const K* __rest
     __syncwarp();
   }
   __syncthreads();
-  for(unsigned d = threadIdx.x; d < (unsigned)kRadix; d += kThreads) {
+  for(unsigned d = threadIdx.x; d < (unsigned)kRadix; d += kScatterThreads) {
     dbase[d] = offsets[(uint64_t)d * nblocks + blockIdx.x];
     uint32_t run = 0;
 #pragma unroll
@@ -290,12 +291,6 @@ struct sort_scratch {
   dev_buf scan;      // scan scratch
 };
 
-// MR_SORT_THREADS=256: the scatter kernel's first shape (A/B switch); default 512 threads x 8 keys
-inline bool sort_wide_ctas() {
-  static const bool v = [] { const char* e = getenv("MR_SORT_THREADS"); return !(e && atoi(e) == 256); }();
-  return v;
-}
-
 // one pass on the digit [shift, shift + kBits)
 template<typename K, typename V, int kBits>
 int radix_pass(mr_context* ctx, const K* kin, const V* vin, K* kout, V* vout, uint64_t n, int shift, sort_scratch& s) {
@@ -304,18 +299,9 @@ int radix_pass(mr_context* ctx, const K* kin, const V* vin, K* kout, V* vout, ui
   radix_hist_kernel<K, kBits><<<nblocks, kSortThreads, 0, ctx->stream>>>(kin, n, shift, s.table.as<uint32_t>(), nblocks);
   MR_LAUNCHED(ctx);
   MR_TRY((exclusive_scan<ptr_in_u32, uint64_t>(ctx, ptr_in_u32{ s.table.as<uint32_t>() }, tsize, s.offsets.as<uint64_t>(), s.scan, nullptr)));
-  if(sort_wide_ctas()) radix_scatter_kernel<K, V, kBits, 512><<<nblocks, 512, 0, ctx->stream>>>(kin, vin, kout, vout, n, shift, s.offsets.as<uint64_t>(), nblocks);
-  else                 radix_scatter_kernel<K, V, kBits, 256><<<nblocks, 256, 0, ctx->stream>>>(kin, vin, kout, vout, n, shift, s.offsets.as<uint64_t>(), nblocks);
+  radix_scatter_kernel<K, V, kBits><<<nblocks, kScatterThreads, 0, ctx->stream>>>(kin, vin, kout, vout, n, shift, s.offsets.as<uint64_t>(), nblocks);
   MR_LAUNCHED(ctx);
   return MR_OK;
-}
-
-// MR_SORT_EVEN_DIGITS=1: equal digits (14 bits as 7 + 7 instead of 8 + 6).  Measured on B200: group sort 13.9 -> 14.9 ms
-// per step on the yeast shape, 446 -> 462 on the human shape -- the shorter runs of 256 buckets cost less than
-// the second pass gains from having only 64 -- so the default is digits of 8 bits, the last one shorter.
-inline bool sort_even_digits() {
-  static const bool v = [] { const char* e = getenv("MR_SORT_EVEN_DIGITS"); return e && atoi(e) == 1; }();
-  return v;
 }
 
 // Sorts (k0,v0) by key bits [lo_bit, hi_bit) ascending, stable.  k1/v1 are same-sized alternates.
@@ -332,8 +318,8 @@ int radix_sort_pairs(mr_context* ctx, K* k0, V* v0, K* k1, V* v1, uint64_t n, in
   const int bits = hi_bit - lo_bit, passes = (bits + kSortBits - 1) / kSortBits;
   int shift = lo_bit;
   for(int p = 0; p < passes; ++p) {
-    // equal digits: the first (bits % passes) passes take one bit more
-    int w = sort_even_digits() ? bits / passes + (p < bits % passes ? 1 : 0) : std::min(kSortBits, hi_bit - shift);
+    // digits of kSortBits bits, the last one narrower: faster than equal digits (DESIGN.md §4)
+    int w = std::min(kSortBits, hi_bit - shift);
     K* kin = first ? k0 : k1; V* vin = first ? v0 : v1;
     K* kout = first ? k1 : k0; V* vout = first ? v1 : v0;
     switch(w) {

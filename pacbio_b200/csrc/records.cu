@@ -655,7 +655,7 @@ int mr_records(mr_context* ctx, const mr_result* res, const mr_records_params* p
     MR_LAUNCHED(ctx);
     MR_TRY((prim::exclusive_scan<prim::ptr_in_u32, uint64_t>(ctx, prim::ptr_in_u32{ A.line_len }, Sc, A.line_off, ws.scan_scratch, d_tot + 1)));
     MR_CUDA(ctx, cudaMemcpyAsync(h, A.err, 24, cudaMemcpyDeviceToHost, st));
-    MR_CUDA(ctx, ctx->wait(st));
+    MR_CUDA(ctx, cudaStreamSynchronize(st));
   }
   if(h[0] != ~0ULL)
     return ctx->fail(MR_EINVAL, (h[0] & 1) ? "unitig id of a super-read name is not in the -u file"
@@ -669,7 +669,7 @@ int mr_records(mr_context* ctx, const mr_result* res, const mr_records_params* p
     emit_lines_kernel<<<div_up(nlines * 32, 256), 256, 0, st>>>(A, nlines);
     MR_LAUNCHED(ctx);
     MR_CUDA(ctx, cudaMemcpyAsync(t->host->p, A.text, bytes, cudaMemcpyDeviceToHost, st));
-    MR_CUDA(ctx, ctx->wait(st));
+    MR_CUDA(ctx, cudaStreamSynchronize(st));
   }
   *out = t.release();
   return MR_OK;

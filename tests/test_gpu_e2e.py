@@ -350,8 +350,7 @@ def test_tiles_staged_without_bulk_copies_give_the_same_records(tmpdir_session, 
 
 
 @pytest.mark.parametrize("env", [{"MR_READ_SORT": "0"}, {"MR_GSORT_CAP": "32"}, {"MR_GSORT_CAP": "256"},
-                                 {"MR_GSORT_THREADS": "1024"}, {"MR_GSORT_THREADS": "1024", "MR_GSORT_CAP": "1024"},
-                                 {"MR_GSORT_BALLOT": "1"}, {"MR_FINISH_QUAD": "1"}])
+                                 {"MR_GSORT_THREADS": "1024"}, {"MR_GSORT_THREADS": "1024", "MR_GSORT_CAP": "1024"}])
 def test_grouping_routes_give_the_same_records(tmpdir_session, tmp_path, env):
     """Hits are grouped by (read, super-read) one CTA per read: in shared memory when the read's hits fit (default for
     these inputs), cut into buckets by the top bits of the super-read index first when they do not, by passes out of
